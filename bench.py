@@ -2,6 +2,7 @@
 """Benchmark of the hot path: render + backward FPS at 1080p, 2.4M Gaussians.
 
   python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload C2|C3|C5] [--colour 3|27|48]
+                  [--dump-outputs DIR]
 
 One "step" = one forward + backward of one 1920x1080 view per GPU: raw parameters ->
 image -> gradients of all five parameter tensors for a fixed upstream image gradient
@@ -321,8 +322,10 @@ def run_ours(args, world, rank, local):
         sampler.start()
     launches0 = None
 
+    last_img = [None]
+
     def step_resident():
-        sc.step(view_id)
+        last_img[0] = sc.step(view_id)
 
     for _ in range(args.warmup):
         step_resident()
@@ -335,6 +338,10 @@ def run_ours(args, world, rank, local):
     e1.record()
     barrier(world)
     launches = gaussian.kernel_launches() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_img[0], {k: getattr(sp.gaussian_3ds, k).grad
+                                                      for k in ("pos", "rgb", "opa", "quat", "scale")})
+    last_img[0] = None
     ms_local = e0.elapsed_time(e1) / args.steps
     ms = max_over_ranks(ms_local, world, dev)
     clocks = sampler.stop() if rank == 0 else {}
@@ -486,6 +493,30 @@ def run_ours(args, world, rank, local):
     if world == 1 and not args.no_cpu_baseline:
         out["cpu_baseline"] = cpu_baseline(args.workload)
     return out
+
+
+DUMP_BYTES = 60 << 20
+
+
+def dump_outputs(out_dir, img, grads):
+    """What the last timed step returned to its caller, as float32 .npy files: `image` (pixels as rows
+    of 3) and `grad_<name>` for each parameter tensor that has a gradient.  So that the dump stays
+    under DUMP_BYTES, arrays longer than k rows keep a fixed sample of k rows (seed 0, one sample per
+    row count, rows in ascending order), k chosen from the bytes of one row of every array."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"image": img.detach().reshape(-1, 3)}
+    arrays.update({"grad_" + k: g for k, g in grads.items() if g is not None})
+    k = DUMP_BYTES // sum(4 * a[0].numel() for a in arrays.values())
+    samples = {}
+    for name, a in arrays.items():
+        n = a.shape[0]
+        if n > k:
+            if n not in samples:
+                perm = torch.randperm(n, generator=torch.Generator().manual_seed(0))
+                samples[n] = perm[:k].sort().values.to(a.device)
+            a = a[samples[n]]
+        np.save(os.path.join(out_dir, name + ".npy"), a.float().cpu().numpy())
 
 
 def _short_leg(sc, steps=10, warmup=3):
@@ -661,7 +692,14 @@ def main():
     ap.add_argument("--colour", type=int, default=3, choices=[3, 27, 48],
                     help="3 = RGB (default; the reference's published 2.4M point), 27 = per-pixel SH degree 2 "
                          "(the reference's use_sh_coeff), 48 = SH degree 3 extension")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the image and parameter gradients of the last timed step to DIR/<name>.npy "
+                         "(float32; large arrays as a fixed seeded sample of rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (the product path has no CPU fallback)")
     if args.impl != "reference":

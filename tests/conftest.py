@@ -43,13 +43,3 @@ def gs(cuda):
     import gaussian   # noqa: F401  built in-tree by 3d-gaussian-splatting_b200/build.py
     import renderer
     return gaussian, renderer
-
-
-@pytest.fixture(scope="session")
-def ref(cuda):
-    """The reference's own CUDA build (oracle/_ref); tests that need it skip if it is absent."""
-    import ref_pipeline
-    g, r = ref_pipeline.load_reference()
-    if g is None:
-        pytest.skip("oracle/_ref reference build not present")
-    return g, r

@@ -2,6 +2,7 @@
 build on a GPU and writes tests/golden/*.npz) and tests/test_oracle.py (checks the CPU
 oracle against those files).  All inputs are regenerated from seeds; the .npz files hold
 the reference's outputs (plus the few inputs that are themselves oracle-derived)."""
+import numpy as np
 import torch
 
 import gs_oracle as O
@@ -80,6 +81,23 @@ def reference_key_collisions(g, cam):
     key = depth + tile * (depth.max() + 1)
     bad = int(((key[1:] <= key[:-1]) & (tile[1:] == tile[:-1])).sum())
     return bad, int(cnt.max()), g["pos"].shape[0] // 20
+
+
+def sample(rows, k, seed=0):
+    """A fixed, seeded sample of at most k entries of the index tensor `rows`.  The first j entries
+    of a sample are the sample for k = j, so a stored sample can be shortened without re-running."""
+    rows = torch.as_tensor(rows).flatten()
+    perm = torch.randperm(rows.numel(), generator=torch.Generator().manual_seed(seed))
+    return rows[perm[:k]]
+
+
+def tile_set_digest(sets):
+    """Per-tile count, sum and sum of squares of the Gaussian ids in each tile's list: equal digests
+    mean equal per-tile sets for any change short of a coincidence in all three."""
+    ids = [torch.tensor(s, dtype=torch.int64) for s in sets]
+    return dict(counts=np.array([i.numel() for i in ids], dtype=np.int32),
+                sum=np.array([int(i.sum()) for i in ids], dtype=np.int64),
+                sum_sq=np.array([int((i * i).sum()) for i in ids], dtype=np.int64))
 
 
 def check_oracle_against(name, gold):

@@ -51,6 +51,22 @@ def load_golden(name):
     return {k: torch.from_numpy(z[k]) for k in z.files}
 
 
+def require_golden(name):
+    """A committed fixture of tests/golden/ (written by tests/golden/make_golden.py); missing is an error."""
+    gold = load_golden(name)
+    assert gold is not None, f"tests/golden/{name} is missing"
+    return gold
+
+
+def assert_matches_golden_frame(sp, img, gold, img_atol, grad_rtol):
+    """A rendered frame and the five parameter gradients of Splatter `sp` against a fixture that
+    holds the image on a pixel sample (`pix`, `image`) and the gradients on a row sample (`rows`)."""
+    assert abs_err(img.detach().reshape(-1, 3).cpu()[gold["pix"].long()], gold["image"]) < img_atol
+    r = gold["rows"].long()
+    for name in ("pos", "rgb", "opa", "quat", "scale"):
+        assert rel_err(getattr(sp.gaussian_3ds, name).grad.cpu()[r], gold["grad_" + name]) < grad_rtol, name
+
+
 def device_depth_keys(g, cam, dev, scale_activation="abs"):
     """float32 depth |p_c| of every Gaussian as the CUDA path computes it (legacy
     `global_culling`, same device function as the fused projection); culled rows are 0.  Used as

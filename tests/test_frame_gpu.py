@@ -1,6 +1,7 @@
 """GPU parity of the fused frame path (parameters -> image -> parameter gradients) against
-the CPU oracle, the committed golden fixtures and the reference build's whole pipeline;
-plus size-independent properties at BASELINE.json's full sizes (P3/P5/P6 of SURVEY.md §8c).
+the CPU oracle, the committed golden fixtures and the reference build's whole pipeline (its
+outputs stored in tests/golden/ref_frame.npz); plus size-independent properties at
+BASELINE.json's full sizes (P3/P5/P6 of SURVEY.md §8c).
 """
 import os
 
@@ -9,7 +10,8 @@ import torch
 
 import gs_oracle as O
 import synthetic as S
-from helpers import abs_err, device_depth_keys, load_golden, rel_err, scene
+from helpers import (abs_err, assert_matches_golden_frame, device_depth_keys, load_golden, rel_err, require_golden,
+                     scene)
 
 pytestmark = pytest.mark.gpu
 
@@ -83,28 +85,19 @@ def test_fused_frame_sh_vs_oracle(gs, cuda, sh_dim, opa, sh_tc):
         gs[0].tune("sh_tc", 3)
 
 
-def test_fused_frame_vs_reference_pipeline(gs, ref, cuda):
+def test_fused_frame_vs_reference_pipeline(gs, cuda):
     """P5: whole reference pipeline (its CUDA build + its renderer.py + the splatter.py call
-    sequence) vs our fused path on a C1-class scene inside the reference's safe regime."""
-    import ref_pipeline
-    gref, rref = ref
+    sequence; outputs in tests/golden/ref_frame.npz) vs our fused path on a C1-class scene inside
+    the reference's safe regime."""
     import golden_cases as GC
     # a scene inside the reference's own limits (capacity MAXP = n//20, no fp32 sort-key ties)
     n, w, h = 2000, 192, 128
     g, v, cam, go = GC.frame_case(n, w, h, (0.005, 0.05), (0.4, 1.5), 2)
     assert GC.reference_key_collisions(g, cam)[0] == 0
-    go = go.to(cuda)
-    frame = ref_pipeline.LegacyFrame(gref, rref, w, h, v.fx, v.fy, v.rot.to(cuda), v.tran.to(cuda))
-    p = {k: t.to(cuda).clone().requires_grad_(True) for k, t in g.items()}
-    rimg = frame(p["pos"], p["rgb"], p["opa"], p["quat"], p["scale"])
-    rimg.backward(go)
-    assert frame.aux["max_tile"] <= min(500, frame.aux["MAXP"])
     sp = _splatter(g, [v], cuda)
     img = sp(0)
-    img.backward(go)
-    assert abs_err(img, rimg) < IMG_ATOL
-    for name in ("pos", "rgb", "opa", "quat", "scale"):
-        assert rel_err(getattr(sp.gaussian_3ds, name).grad, p[name].grad) < GRAD_RTOL, name
+    img.backward(go.to(cuda))
+    assert_matches_golden_frame(sp, img, require_golden("ref_frame.npz"), IMG_ATOL, GRAD_RTOL)
 
 
 def test_legacy_boundary_drop_in(gs, cuda):

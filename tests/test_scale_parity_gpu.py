@@ -4,25 +4,24 @@ epoch-tagged tails of the gradient rows are skipped:
 
 * `test_p4_at_c2`        - C2 (500 k Gaussians, 1080p): the reference build's own `draw` /
                            `draw_backward` (through its unmodified renderer.py) fed OUR sorted
-                           per-instance order; image and all five parameter gradients vs the fused path.
+                           per-instance order; image and all five parameter gradients vs the fused path
+                           (the reference's outputs are stored in tests/golden/ref_p4_c2_*.npz).
 * `test_masked_gradient_at_scale` - C3 (2.4 M, 1080p; RGB, SH-27, SH-48) and C5 (5 M, 4K): the upstream
                            gradient is non-zero only on K sampled tiles (the heaviest tile, the most
                            saturated one, a spread); ALL FIVE parameter gradients are compared with the
                            fp64 CPU oracle run on exactly the Gaussians of those tiles, every other
                            gradient must be exactly zero.
 * `test_reference_renderer_bound_to_our_module` - the reference's renderer.py, UNCHANGED, imported
-                           with `gaussian` = our extension (SURVEY.md §2 #5), incl. a strided grad_output.
+                           with `gaussian` = our extension (SURVEY.md §2 #5), incl. a strided grad_output
+                           (its outputs are stored in tests/golden/ref_renderer_*.npz).
 """
-import importlib.util
-import os
-import sys
-
+import numpy as np
 import pytest
 import torch
 
 import gs_oracle as O
 import synthetic as S
-from helpers import abs_err, rel_err, scene
+from helpers import abs_err, assert_matches_golden_frame, rel_err, require_golden, scene
 
 pytestmark = pytest.mark.gpu
 
@@ -38,25 +37,6 @@ def _splatter(g, views, dev, **kw):
 
 
 # ------------------------------------------------------------------------------------------
-def _reference_chain(rref, g, v, cam, gi, accum, go, dev):
-    """The reference's own operators (its CUDA build through its unmodified renderer.py) on OUR sorted
-    instance order: pre-activations (splatter.py:519-524,539-540) -> global_culling -> gather (a8) ->
-    draw -> clamp + crop (splatter.py:652-653) -> backward of all of it."""
-    p = {k: t.to(dev).clone().requires_grad_(True) for k, t in g.items()}
-    nq = p["quat"] / p["quat"].norm(dim=1, keepdim=True)
-    ns = p["scale"].abs() + 1e-4
-    _pos, _cov, mask = rref.global_culling(p["pos"], nq, ns, v.rot.to(dev), v.tran.to(dev), cam.near,
-                                           cam.half_w, cam.half_h)
-    t_pos, t_cov = _pos[gi], _cov[gi]
-    t_rgb, t_opa = p["rgb"].sigmoid()[gi], p["opa"].sigmoid()[gi]
-    dummy = torch.zeros(3, device=dev)
-    rimg_p = rref.draw(t_pos, t_rgb, t_opa, t_cov, accum, cam.Hp, cam.Wp, cam.fx, cam.fy, False, False, False, True,
-                       dummy, dummy, dummy, dummy)
-    rimg = cam.crop(torch.clamp(rimg_p, 0, 1))
-    rimg.backward(go)
-    return rimg.detach(), {k: p[k].grad for k in NAMES}, mask
-
-
 def _tile_mask(cam, tiles, h, w):
     top, left = (cam.Hp - h) // 2, (cam.Wp - w) // 2
     mpad = torch.zeros(cam.Hp, cam.Wp, 1)
@@ -67,52 +47,55 @@ def _tile_mask(cam, tiles, h, w):
 
 
 @pytest.mark.parametrize("regime,opa", [("safe", (0.005, 0.05)), ("standard", (0.05, 0.9))])
-def test_p4_at_c2(gs, ref, cuda, regime, opa):
+def test_p4_at_c2(gs, cuda, regime, opa):
     """SURVEY.md §8c "P4@C2": C2 (500 k Gaussians, 1080p; heaviest tile <= 500 instances, inside the limit
     below which the reference's draw_backward does not mix chunks - hazard 1).  The reference build's own
-    kernels are fed OUR (tile, depth, id) order, so its fp32 sort-key ties (hazard 4) cannot enter.
+    kernels were fed OUR (tile, depth, id) order, so its fp32 sort-key ties (hazard 4) cannot enter; what
+    they computed is tests/golden/ref_p4_c2_<regime>.npz (culling mask, image on a pixel sample, gradients
+    on a sample of rows).
       safe     - opacities in [0.005, 0.05]: no pixel reaches T < 1e-4, the reference's backward is exact:
                  image <= 1e-4 and ALL gradients <= 1e-3 are gated against it;
       standard - the benchmark's opacities [0.05, 0.9]: pixels saturate, and the reference's partial-mask
                  shuffle reduction (hazard 3, gaussian.cu:675-772) is no longer exact.  The image is gated
                  against the reference; for the gradients the fp64 oracle arbitrates on sampled tiles: ours
                  must match it to 1e-3, and any disagreement with the reference must be the reference's."""
-    gref, rref = ref
+    gold = require_golden(f"ref_p4_c2_{regime}.npz")
     n, w, h = 500_000, 1920, 1080
     g, v, cam = scene(n, w, h, k=0, opa_range=opa)
     go = (S.make_grad_output(h, w, 0) * (h * w)).to(cuda)
     sp = _splatter(g, [v], cuda)
     img = sp(0)
     img.backward(go)
-    ours = {k: getattr(sp.gaussian_3ds, k).grad.clone() for k in NAMES}
     st = sp.frame_stats()
     assert st["max_tile_count"] <= 500, st
     idx, accum = sp._rctx.sorted_instances()
-    gi = idx.long()
-    rimg, rgrads, mask = _reference_chain(rref, g, v, cam, gi, accum, go, cuda)
-    assert torch.equal(mask, sp.culling_mask)
-    assert abs_err(img, rimg) < IMG_ATOL
-    errs = {k: rel_err(ours[k], rgrads[k]) for k in NAMES}
-    print(f"P4@C2[{regime}] ours vs reference build, full frame: {errs}")
+    mask = torch.from_numpy(np.unpackbits(gold["mask"].numpy(), count=n).astype(bool))
+    assert torch.equal(sp.culling_mask.cpu().bool(), mask)
+    assert abs_err(img.detach().reshape(-1, 3).cpu()[gold["pix"].long()], gold["image"]) < IMG_ATOL
+    r = gold["rows"].long()
+    errs = {k: rel_err(getattr(sp.gaussian_3ds, k).grad.cpu()[r], gold["grad_" + k]) for k in NAMES}
+    print(f"P4@C2[{regime}] ours vs reference build, sampled rows: {errs}")
     if regime == "safe":
         assert st["n_instances_eff"] == st["n_instances"]              # nothing saturated
         for k in NAMES:
             assert errs[k] < GRAD_RTOL, (k, errs)
         return
-    # standard regime: arbitrate on sampled tiles with the fp64 oracle
-    neff = sp._rctx.tile_consumed().cpu().long()
-    tiles = _pick_tiles(accum.cpu().long(), neff, cam.ntx, cam.nty, 5)
+    # standard regime: arbitrate on the fixture's tiles with the fp64 oracle
+    tiles = gold["tiles"].tolist()
     gom = S.make_grad_output(h, w, 0) * (h * w) * _tile_mask(cam, tiles, h, w)
     for p_ in sp.gaussian_3ds.parameters():
         p_.grad = None
     sp(0).backward(gom.to(cuda))
-    _, rg, _ = _reference_chain(rref, g, v, cam, gi, accum, gom.to(cuda), cuda)
     _, U, og = _oracle_on_tiles(g, v, cam, idx.cpu(), accum.cpu().long(), tiles, gom, False)
+    # the reference's gradients are stored for a sample of the Gaussians binned into those tiles
+    u_ids = gold["u_ids"].long()
+    loc = torch.searchsorted(U, u_ids).clamp(max=U.numel() - 1)
+    assert torch.equal(U[loc], u_ids)
     for k in NAMES:
         e_ours = rel_err(getattr(sp.gaussian_3ds, k).grad.cpu()[U], og[k])
-        e_ref = rel_err(rg[k].cpu()[U], og[k])
-        print(f"P4@C2[standard] {k}: ours vs oracle {e_ours:.2e}, reference vs oracle {e_ref:.2e}, "
-              f"ours vs reference (full frame) {errs[k]:.2e}")
+        e_ref = rel_err(gold["tiles_grad_" + k], og[k][loc])
+        print(f"P4@C2[standard] {k}: ours vs oracle {e_ours:.2e}, reference vs oracle (sampled) {e_ref:.2e}, "
+              f"ours vs reference (sampled rows) {errs[k]:.2e}")
         assert e_ours < GRAD_RTOL, (k, e_ours)
         assert errs[k] < GRAD_RTOL or e_ref > 10 * e_ours, (k, errs[k], e_ref, e_ours)
 
@@ -203,37 +186,13 @@ def test_masked_gradient_at_scale(gs, cuda, label, n, w, h, sh_dim):
 
 
 # ------------------------------------------------------------------------------------------
-def _reference_renderer_on(gmod):
-    """The reference's renderer.py (oracle/_ref/renderer.py, byte-identical copy made by
-    oracle/build_ref.py), imported with `gaussian` bound to `gmod`."""
-    import ref_pipeline
-    rpy = os.path.join(ref_pipeline.REF_DIR, "renderer.py")
-    if not os.path.exists(rpy):
-        pytest.skip("oracle/_ref/renderer.py not present")
-    saved = sys.modules.get("gaussian")
-    sys.modules["gaussian"] = gmod
-    try:
-        spec = importlib.util.spec_from_file_location("renderer_ref_on_ours", rpy)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-    finally:
-        if saved is None:
-            del sys.modules["gaussian"]
-        else:
-            sys.modules["gaussian"] = saved
-    return mod
-
-
 @pytest.mark.parametrize("use_sh", [False, True])
 def test_reference_renderer_bound_to_our_module(gs, cuda, use_sh):
-    """SURVEY.md §2 #5 / §8b: reference renderer.py runs UNCHANGED on our `gaussian` module, driven by
-    the reference's splatter.py call sequence (oracle/ref_pipeline.LegacyFrame), and agrees with the
-    fused path; the upstream gradient is a strided (non-contiguous) view."""
+    """SURVEY.md §2 #5 / §8b: the reference's renderer.py, UNCHANGED, driven by the reference's splatter.py
+    call sequence (oracle/ref_pipeline.LegacyFrame) with `gaussian` bound to our module and a strided
+    (non-contiguous) upstream gradient; what it computed is tests/golden/ref_renderer_{rgb,sh}.npz.
+    The fused path must agree with it."""
     import golden_cases as GC
-    import ref_pipeline
-    gaussian, _ = gs
-    rmod = _reference_renderer_on(gaussian)
-    assert rmod.gaussian is gaussian and "oracle" in rmod.__file__
     n, w, h = 2000, 192, 128
     # a scene inside the reference pipeline's own limits (capacity n//20, no fp32 sort-key ties); the
     # SH variant has the same geometry (the generator draws colours last)
@@ -241,19 +200,8 @@ def test_reference_renderer_bound_to_our_module(gs, cuda, use_sh):
     assert GC.reference_key_collisions(g, cam)[0] == 0
     if use_sh:
         g, v, cam = scene(n, w, h, seed=6, sh_dim=27, opa_range=(0.05, 0.6), sigma_px=(0.4, 1.5))
-    wide = torch.zeros(h, w, 6, device=cuda)
-    wide[..., ::2] = go.to(cuda)
-    go_strided = wide[..., ::2]
-    assert not go_strided.is_contiguous()
-    frame = ref_pipeline.LegacyFrame(gaussian, rmod, w, h, v.fx, v.fy, v.rot.to(cuda), v.tran.to(cuda),
-                                     use_sh_coeff=use_sh)
-    p = {k: t.to(cuda).clone().requires_grad_(True) for k, t in g.items()}
-    limg = frame(p["pos"], p["rgb"], p["opa"], p["quat"], p["scale"])
-    assert frame.aux["max_tile"] <= frame.aux["MAXP"]
-    limg.backward(go_strided)
     sp = _splatter(g, [v], cuda, use_sh_coeff=use_sh)
     img = sp(0)
     img.backward(go.to(cuda))
-    assert abs_err(img, limg) < IMG_ATOL
-    for name in NAMES:
-        assert rel_err(getattr(sp.gaussian_3ds, name).grad, p[name].grad) < GRAD_RTOL, name
+    gold = require_golden(f"ref_renderer_{'sh' if use_sh else 'rgb'}.npz")
+    assert_matches_golden_frame(sp, img, gold, IMG_ATOL, GRAD_RTOL)

@@ -1,15 +1,18 @@
 """GPU parity of the legacy per-stage boundary (the reference's `gaussian` module surface)
-against the CPU oracle and, when oracle/_ref is present, against the reference's own CUDA
-build on identical inputs.  Protocol P1/P2/P4 of SURVEY.md §8c.
+against the CPU oracle and against the reference's own CUDA build on identical inputs (its
+outputs stored in tests/golden/ref_*.npz by tests/golden/make_golden.py).  Protocol P1/P2/P4
+of SURVEY.md §8c.
 
 Tolerances (BASELINE.json north_star): image <= 1e-4 abs per pixel; gradients <= 1e-3
 relative (max |delta| / max |reference| per tensor); projection 1e-5 relative.
 """
+import numpy as np
 import pytest
 import torch
 
+import golden_cases as GC
 import gs_oracle as O
-from helpers import abs_err, rel_err, scene, sorted_instances_cpu
+from helpers import abs_err, rel_err, require_golden, scene, sorted_instances_cpu
 
 pytestmark = pytest.mark.gpu
 
@@ -61,29 +64,29 @@ def test_global_culling_forward_backward_vs_oracle(gs, cuda, k):
         assert float(op[culled].abs().max()) == 0 and float(pos.grad[culled].abs().max()) == 0
 
 
-def test_global_culling_vs_reference_build(gs, ref, cuda):
+def test_global_culling_vs_reference_build(gs, cuda):
+    """Against the reference build's outputs on the same inputs (tests/golden/ref_culling.npz: the
+    full mask, everything else on a sample of visible rows)."""
     gaussian, renderer = gs
-    gref, rref = ref
+    gold = require_golden("ref_culling.npz")
     g, cam, nq, ns = _proj_inputs(20000, 640, 360, 1, cuda)
-    args = (cam.rot.to(cuda), cam.tran.to(cuda), cam.near, cam.half_w, cam.half_h)
-    outs = []
-    for R in (renderer, rref):
-        pos = g["pos"].to(cuda).requires_grad_(True)
-        q = nq.to(cuda).requires_grad_(True)
-        s = ns.to(cuda).requires_grad_(True)
-        op, oc, om = R.global_culling(pos, q, s, *args)
-        gen = torch.Generator().manual_seed(3)
-        gp = torch.randn(op.shape, generator=gen).to(cuda)
-        gc = torch.randn(oc.shape, generator=gen).to(cuda)
-        ((op * gp).sum() + (oc * gc).sum()).backward()
-        outs.append((op, oc, om, pos.grad, q.grad, s.grad))
-    a, b = outs
-    assert torch.equal(a[2], b[2])
+    pos = g["pos"].to(cuda).requires_grad_(True)
+    q = nq.to(cuda).requires_grad_(True)
+    s = ns.to(cuda).requires_grad_(True)
+    op, oc, om = renderer.global_culling(pos, q, s, cam.rot.to(cuda), cam.tran.to(cuda), cam.near, cam.half_w,
+                                         cam.half_h)
+    gen = torch.Generator().manual_seed(3)
+    gp = torch.randn(op.shape, generator=gen).to(cuda)
+    gc = torch.randn(oc.shape, generator=gen).to(cuda)
+    ((op * gp).sum() + (oc * gc).sum()).backward()
+    assert torch.equal(om.cpu().bool(), gold["mask"])
+    r = gold["rows"].long()
+    a = [t.detach().cpu()[r] for t in (op, oc, pos.grad, q.grad, s.grad)]
     # depth (the sort key) is bit-identical to the reference kernel's: same ordering keys
-    assert torch.equal(a[0][:, 2], b[0][:, 2])
-    assert rel_err(a[0], b[0]) < 1e-5 and rel_err(a[1], b[1]) < 2e-5
-    for i in (3, 4, 5):
-        assert rel_err(a[i], b[i]) < 1e-4
+    assert torch.equal(a[0][:, 2], gold["res_pos"][:, 2])
+    assert rel_err(a[0], gold["res_pos"]) < 1e-5 and rel_err(a[1], gold["res_cov"]) < 2e-5
+    for x, k in zip(a[2:], ("grad_pos", "grad_quat", "grad_scale")):
+        assert rel_err(x, gold[k]) < 1e-4, k
 
 
 def _tile_lists(gmod, pos, cov, cam, dev, thresh=0.05, maxp=None):
@@ -141,17 +144,20 @@ def test_tile_binning_and_gather_vs_oracle(gs, cuda):
         assert bool((tid[s:e] == t).all())
 
 
-def test_tile_binning_vs_reference_build(gs, ref, cuda):
+def _assert_same_sets(sets, gold, prefix=""):
+    """Per-tile sets equal to the reference build's, compared through GC.tile_set_digest."""
+    for k, a in GC.tile_set_digest(sets).items():
+        assert np.array_equal(a, gold[prefix + k].numpy()), prefix + k
+
+
+def test_tile_binning_vs_reference_build(gs, cuda):
     gaussian, _ = gs
-    gref, _ = ref
     g, v, cam = scene(30000, 640, 368, k=0)
     nq, ns, _, _ = O.preactivate(g["quat"], g["scale"], g["opa"], g["rgb"])
     rp, rc, m = O.global_culling(g["pos"], nq, ns, cam.rot, cam.tran, cam.near, cam.half_w, cam.half_h)
     idx = torch.nonzero(m.bool()).squeeze(-1)
     pos, cov = rp[idx].contiguous(), rc[idx].contiguous()
-    a = _per_tile_sets(*_tile_lists(gaussian, pos, cov, cam, cuda))
-    b = _per_tile_sets(*_tile_lists(gref, pos, cov, cam, cuda))
-    assert a == b
+    _assert_same_sets(_per_tile_sets(*_tile_lists(gaussian, pos, cov, cam, cuda)), require_golden("ref_tiles.npz"))
 
 
 def _draw_case(n, w, h, opa_range, seed=0):
@@ -198,20 +204,24 @@ def test_draw_forward_backward_vs_oracle(gs, cuda, case):
     assert float(grads["pos"][:, 2].abs().max()) == 0.0      # depth: sort key only
 
 
-def test_draw_vs_reference_build_safe_regime(gs, ref, cuda):
-    """P4: identical sorted inputs to both extensions, inside the reference's safe regime
-    (per-tile count <= 500, no pixel reaching T < 1e-4; SURVEY.md §8c hazards 1-3)."""
+def _assert_matches_reference_draw(img, grads, gold):
+    """Image on the stored pixel sample, gradients on the stored instance sample."""
+    assert abs_err(img.reshape(-1, 3).cpu()[gold["pix"].long()], gold["image"]) < IMG_ATOL
+    r = gold["rows"].long()
+    for k in ("rgb", "opa", "cov"):
+        assert rel_err(grads[k].cpu()[r], gold["grad_" + k]) < GRAD_RTOL, k
+    assert rel_err(grads["pos"][:, :2].cpu()[r], gold["grad_pos"]) < GRAD_RTOL
+
+
+def test_draw_vs_reference_build_safe_regime(gs, cuda):
+    """P4: the sorted inputs the reference build was given (tests/golden/ref_draw.npz holds its
+    outputs), inside its safe regime (per-tile count <= 500, no pixel reaching T < 1e-4;
+    SURVEY.md §8c hazards 1-3)."""
     _, renderer = gs
-    _, rref = ref
     cam, inst, gi = _draw_case(4000, 256, 256, (0.005, 0.05))
     counts = inst["accum"][1:] - inst["accum"][:-1]
     assert int(counts.max()) <= 500
-    a_img, a_g = _run_draw(renderer, inst, cam, gi, cuda)
-    b_img, b_g = _run_draw(rref, inst, cam, gi, cuda)
-    assert abs_err(a_img, b_img) < IMG_ATOL
-    for k in ("rgb", "opa", "cov"):
-        assert rel_err(a_g[k], b_g[k]) < GRAD_RTOL, k
-    assert rel_err(a_g["pos"][:, :2], b_g["pos"][:, :2]) < GRAD_RTOL
+    _assert_matches_reference_draw(*_run_draw(renderer, inst, cam, gi, cuda), require_golden("ref_draw.npz"))
 
 
 def test_draw_edge_cases(gs, cuda):
@@ -289,19 +299,15 @@ def test_draw_sh_forward_backward_vs_oracle(gs, cuda, sh_dim, case):
     assert rel_err(grads["pos"][:, :2], t["pos"].grad[:, :2]) < GRAD_RTOL
 
 
-def test_draw_sh_vs_reference_build(gs, ref, cuda):
-    """P4 for SH-27 inside the reference's safe regime (<= 160 instances per tile in backward)."""
+def test_draw_sh_vs_reference_build(gs, cuda):
+    """P4 for SH-27 inside the reference's safe regime (<= 160 instances per tile in backward);
+    the reference build's outputs are tests/golden/ref_draw_sh.npz."""
     _, renderer = gs
-    _, rref = ref
     cam, inst, gi, rays = _sh_case(2500, 256, 192, 27, (0.005, 0.05))
     counts = inst["accum"][1:] - inst["accum"][:-1]
     assert int(counts.max()) <= 160
-    a_img, a_g = _run_draw_sh(renderer, inst, cam, gi, rays, cuda)
-    b_img, b_g = _run_draw_sh(rref, inst, cam, gi, rays, cuda)
-    assert abs_err(a_img, b_img) < IMG_ATOL
-    for k in ("rgb", "opa", "cov"):
-        assert rel_err(a_g[k], b_g[k]) < GRAD_RTOL, k
-    assert rel_err(a_g["pos"][:, :2], b_g["pos"][:, :2]) < GRAD_RTOL
+    _assert_matches_reference_draw(*_run_draw_sh(renderer, inst, cam, gi, rays, cuda),
+                                   require_golden("ref_draw_sh.npz"))
 
 
 # ---- legacy tile-culling methods 0 ("dist") and 1 ("prob"): brute force over (Gaussian, tile) ----
@@ -364,10 +370,9 @@ def test_tile_methods_dist_and_prob_vs_torch(gs, cuda):
     assert sum(map(len, want1)) > 0 and flips1 <= 2
 
 
-def test_tile_methods_dist_and_prob_vs_reference_build(gs, ref, cuda):
+def test_tile_methods_dist_and_prob_vs_reference_build(gs, cuda):
     gaussian, _ = gs
-    gref, _ = ref
+    gold = require_golden("ref_tile_methods.npz")
     pos, cov, cam = _small_projected_scene()
     for method, thresh in ((0, (cam.tile_lx / 0.5) ** 2), (1, 0.05)):
-        assert _legacy_lists(gaussian, method, pos, cov, cam, thresh, cuda) == \
-            _legacy_lists(gref, method, pos, cov, cam, thresh, cuda), method
+        _assert_same_sets(_legacy_lists(gaussian, method, pos, cov, cam, thresh, cuda), gold, f"m{method}_")
