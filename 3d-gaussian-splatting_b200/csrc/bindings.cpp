@@ -396,6 +396,79 @@ struct RenderContext {
              "gs_render_backward");
   }
 
+  // depth / alpha maps + background (gs_render_forward_maps): returns [image, depth, alpha, image_raw, depth_raw,
+  // alpha_raw, mask]; with final = false the first three are the raw padded planes themselves
+  std::vector<torch::Tensor> forward_maps(torch::Tensor pos, torch::Tensor rgb, torch::Tensor opa, torch::Tensor quat,
+                                          torch::Tensor scale, int width, int height, float fx, float fy,
+                                          torch::Tensor rot, torch::Tensor tran, float near, float thresh,
+                                          int scale_activation, c10::optional<std::vector<double>> background,
+                                          bool final_layout) {
+    GS_CHECK_F32(pos); GS_CHECK_F32(rgb); GS_CHECK_F32(opa); GS_CHECK_F32(quat); GS_CHECK_F32(scale);
+    int64_t n = pos.size(0);
+    TORCH_CHECK(pos.dim() == 2 && pos.size(1) == 3 && opa.numel() == n && quat.numel() == n * 4 &&
+                    scale.numel() == n * 3 && rgb.dim() == 2 && rgb.size(0) == n && n < (int64_t(1) << 31),
+                "RenderContext.forward_maps: bad shapes");
+    TORCH_CHECK(pos.device().index() == device, "RenderContext was created on another device");
+    float bg[3] = {0.f, 0.f, 0.f};
+    if (background) {
+      TORCH_CHECK(background->size() == 3, "RenderContext.forward_maps: background must have 3 values (r, g, b)");
+      for (int k = 0; k < 3; ++k) bg[k] = (float)(*background)[k];
+    }
+    c10::cuda::CUDAGuard guard(pos.device());
+    gs_camera cam = make_cam(width, height, fx, fy, rot, tran, near, thresh);
+    int wp = (width + 15) / 16 * 16, hp = (height + 15) / 16 * 16;
+    auto raw = torch::empty({hp, wp, 3}, pos.options());
+    auto dpad = torch::empty({hp, wp}, pos.options());
+    auto araw = torch::empty({hp, wp}, pos.options());
+    torch::Tensor fin = raw, dfin = dpad, afin = araw;
+    if (final_layout) {
+      fin = torch::empty({height, width, 3}, pos.options());
+      dfin = torch::empty({height, width}, pos.options());
+      afin = torch::empty({height, width}, pos.options());
+    }
+    auto mask = torch::empty({n}, pos.options().dtype(at::kLong));
+    check_rc(gs_render_forward_maps(ctx, fp(pos), fp(rgb), fp(opa), fp(quat), fp(scale), (int)n, (int)rgb.size(1),
+                                    scale_activation, &cam, bg, fpm(raw), fpm(dpad), fpm(araw),
+                                    final_layout ? fpm(fin) : nullptr, final_layout ? fpm(dfin) : nullptr,
+                                    final_layout ? fpm(afin) : nullptr, mask.data_ptr<int64_t>(), cur_stream()),
+             "gs_render_forward_maps");
+    ++frame;
+    return {fin, dfin, afin, raw, dpad, araw, mask};
+  }
+
+  void backward_maps_into(torch::Tensor pos, torch::Tensor rgb, torch::Tensor opa, torch::Tensor quat,
+                          torch::Tensor scale, torch::Tensor raw, torch::Tensor depth_raw, torch::Tensor alpha_raw,
+                          torch::Tensor grad_image, torch::Tensor grad_depth, torch::Tensor grad_alpha, bool grad_is_final,
+                          torch::Tensor g_pos, torch::Tensor g_rgb, torch::Tensor g_opa, torch::Tensor g_quat,
+                          torch::Tensor g_scale, int64_t expected_frame) {
+    check_frame(expected_frame, "RenderContext.backward_maps_into");
+    GS_CHECK_F32(pos); GS_CHECK_F32(rgb); GS_CHECK_F32(opa); GS_CHECK_F32(quat); GS_CHECK_F32(scale);
+    GS_CHECK_F32(raw); GS_CHECK_F32(depth_raw); GS_CHECK_F32(alpha_raw);
+    GS_CHECK_F32(g_pos); GS_CHECK_F32(g_rgb); GS_CHECK_F32(g_opa); GS_CHECK_F32(g_quat); GS_CHECK_F32(g_scale);
+    TORCH_CHECK(raw.dim() == 3 && raw.size(2) == 3 && depth_raw.dim() == 2 && depth_raw.size(0) == raw.size(0) &&
+                    depth_raw.size(1) == raw.size(1) && alpha_raw.sizes() == depth_raw.sizes(),
+                "RenderContext.backward_maps_into: raw planes must be [Hp,Wp,3], [Hp,Wp], [Hp,Wp]");
+    for (const torch::Tensor* t : {&grad_image, &grad_depth, &grad_alpha})
+      TORCH_CHECK(t->is_cuda() && t->scalar_type() == at::kFloat,
+                  "RenderContext.backward_maps_into: gradients must be float32 CUDA tensors");
+    TORCH_CHECK(grad_image.dim() == 3 && grad_image.size(2) == 3 && grad_depth.dim() == 2 &&
+                    grad_depth.size(0) == grad_image.size(0) && grad_depth.size(1) == grad_image.size(1) &&
+                    grad_alpha.sizes() == grad_depth.sizes(),
+                "RenderContext.backward_maps_into: gradients must be [H,W,3], [H,W], [H,W]");
+    TORCH_CHECK(grad_is_final || grad_image.sizes() == raw.sizes(),
+                "RenderContext.backward_maps_into: padded gradients must match the raw planes");
+    TORCH_CHECK(g_pos.numel() == pos.numel() && g_rgb.numel() == rgb.numel() && g_opa.numel() == opa.numel() &&
+                    g_quat.numel() == quat.numel() && g_scale.numel() == scale.numel(),
+                "RenderContext.backward_maps_into: gradient buffers must match their parameters");
+    TORCH_CHECK(reinterpret_cast<uintptr_t>(g_quat.data_ptr()) % 16 == 0, "grad_quat must be 16-byte aligned");
+    c10::cuda::CUDAGuard guard(pos.device());
+    auto gi = grad_image.contiguous(), gd = grad_depth.contiguous(), ga = grad_alpha.contiguous();
+    check_rc(gs_render_backward_maps(ctx, fp(pos), fp(rgb), fp(opa), fp(quat), fp(scale), fp(raw), fp(depth_raw),
+                                     fp(alpha_raw), fp(gi), fp(gd), fp(ga), grad_is_final ? 1 : 0, fpm(g_pos),
+                                     fpm(g_rgb), fpm(g_opa), fpm(g_quat), fpm(g_scale), cur_stream()),
+             "gs_render_backward_maps");
+  }
+
   int64_t last_instances() { return (int64_t)gs_frame_instances(ctx); }
 
   py::dict stats() {
@@ -598,6 +671,15 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
            py::arg("opa"), py::arg("quat"), py::arg("scale"), py::arg("raw"), py::arg("grad_final"),
            py::arg("g_pos"), py::arg("g_rgb"), py::arg("g_opa"), py::arg("g_quat"), py::arg("g_scale"),
            py::arg("expected_frame") = -1)
+      .def("forward_maps", &RenderContext::forward_maps, py::arg("pos"), py::arg("rgb"), py::arg("opa"),
+           py::arg("quat"), py::arg("scale"), py::arg("width"), py::arg("height"), py::arg("fx"), py::arg("fy"),
+           py::arg("rot"), py::arg("tran"), py::arg("near"), py::arg("thresh"), py::arg("scale_activation"),
+           py::arg("background") = py::none(), py::arg("final") = true)
+      .def("backward_maps_into", &RenderContext::backward_maps_into, py::arg("pos"), py::arg("rgb"), py::arg("opa"),
+           py::arg("quat"), py::arg("scale"), py::arg("raw"), py::arg("depth_raw"), py::arg("alpha_raw"),
+           py::arg("grad_image"), py::arg("grad_depth"), py::arg("grad_alpha"), py::arg("grad_is_final"),
+           py::arg("g_pos"), py::arg("g_rgb"), py::arg("g_opa"), py::arg("g_quat"), py::arg("g_scale"),
+           py::arg("expected_frame") = -1)
       .def("frame_id", &RenderContext::frame_id)
       .def("last_instances", &RenderContext::last_instances)
       .def("stats", &RenderContext::stats)
@@ -620,6 +702,12 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("adam_step", &adam_step, "fused Adam over flat parameter / gradient buffers (CUDA)");
   m.def("tune", [](const std::string& name, int value) { check_rc(gs_tune(name.c_str(), value), "gs_tune"); },
         "set an A/B tuning knob of the blend kernels (see include/gs_b200.h gs_tune)");
+  m.def("tuned", [](const std::string& name) {
+          int v = 0;
+          check_rc(gs_tune_get(name.c_str(), &v), "gs_tune_get");
+          return v;
+        },
+        "current value of an A/B tuning knob of the blend kernels");
   m.def("kernel_launches", []() { return (int64_t)gs_kernel_launches(); },
         "kernels of libgs_b200 launched by this process so far");
   m.attr("abi_version") = gs_abi_version();

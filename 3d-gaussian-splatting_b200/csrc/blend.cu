@@ -3,7 +3,8 @@
 // Semantics: reference gaussian.cu:806-970 (draw_kernel) and :440-803 (draw_backward_kernel):
 // 16x16 pixel tiles, each tile blends its (depth-sorted) instance range front to back,
 // a pixel stops before an instance once its transmittance is < 1e-4, no alpha clamp, no
-// 1/255 skip, black background.  Design (not the reference's):
+// 1/255 skip, black background (the MAPS instantiations of the gather path - an extension - also write depth and
+// alpha maps and composite over a background colour; DESIGN.md §9).  Design (not the reference's):
 //   * each tile's range is contiguous in three packed record streams (see gs_common.cuh) and is
 //     staged into shared memory by 1-D bulk async copies (cp.async.bulk -> UBLKCP, mbarrier
 //     complete_tx), double buffered; one elected thread issues, nobody spends LSU slots on it;
@@ -67,6 +68,7 @@ struct StageView<false> {
   __device__ __forceinline__ float2 b(int j) const { return B[j]; }
   __device__ __forceinline__ float4 c(int j) const { return C[j]; }                   // r, g, b, (slot)
   __device__ __forceinline__ uint32_t slot(int j, int, int) const { return __float_as_uint(C[j].w); }
+  __device__ __forceinline__ float depth(int) const { return 0.f; }                    // not staged (maps: gather only)
 };
 template <>
 struct StageView<true> {
@@ -81,6 +83,7 @@ struct StageView<true> {
     const float4 t = R[j * recw + 1];
     return make_float4(t.z, t.w, R[j * recw + 2].x, 0.f);
   }
+  __device__ __forceinline__ float depth(int j) const { return R[j * recw + 2].y; }   // |p_c| (maps frames)
   // gradient row of this (Gaussian, tile) instance: first row of the Gaussian + rank of the tile in its rectangle
   __device__ __forceinline__ uint32_t slot(int j, int tx, int ty) const {
     const float4 cc = R[j * recw + 2];
@@ -138,7 +141,10 @@ __device__ __forceinline__ void gather_issue(SM& sm, int stage, const GsRec* __r
 // Per (thread, instance): 3 broadcast LDS + 4 row-shared FP32 ops (dy, cb*dy, cc*dy, l2o-cc*dy^2)
 // + 4 pixels x (dx, u, exponent, MUFU.EX2, setp, mul, sel, 3 FFMA colour, T update) = 12.75
 // issue slots per (pixel, instance) instead of 17-18 with one pixel per thread.
-template <int FWD_CH, int PX, bool GATHER>
+// MAPS (gather path only): one more FFMA per (pixel, instance) accumulates the depth map; the epilogue adds T * bg to
+// the colour and stores depth and alpha = 1 - T.  `maps` is the last parameter so that the other instantiations keep
+// their parameter offsets (and their code).
+template <int FWD_CH, int PX, bool GATHER, bool MAPS = false>
 __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __restrict__ pA,
                                                                  const float2* __restrict__ pB,
                                                                  const float4* __restrict__ pC,
@@ -148,7 +154,9 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
                                                                  int ntx, float fx, float fy,
                                                                  float* __restrict__ image,
                                                                  int* __restrict__ tile_neff,
-                                                                 float* __restrict__ final_img, GsCrop crop) {
+                                                                 float* __restrict__ final_img, GsCrop crop,
+                                                                 GsMapsFwd maps = GsMapsFwd{}) {
+  static_assert(!MAPS || GATHER, "depth / alpha maps read the depth from the gathered records");
   using Smem = typename std::conditional<GATHER, GatherRing<FWD_CH, FWD_STAGES, 3>, FwdSmem<FWD_CH>>::type;
   __shared__ __align__(16) Smem sm;
   const int tile = blockIdx.x;
@@ -186,10 +194,12 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
   }
 
   float T[FWD_PX], cr[FWD_PX], cg[FWD_PX], cb[FWD_PX];
+  float dd[FWD_PX];                                   // depth map (MAPS only)
 #pragma unroll
   for (int p = 0; p < FWD_PX; ++p) {
     T[p] = 1.f;
     cr[p] = cg[p] = cb[p] = 0.f;
+    dd[p] = 0.f;
   }
   int consumed = cnt;
   int k = 0;
@@ -212,6 +222,8 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
     const float4 a = sv.a(J);                                                               \
     const float2 b = sv.b(J);                                                               \
     const float4 c = sv.c(J);                                                               \
+    float dep = 0.f;                                                                        \
+    if constexpr (MAPS) dep = sv.depth(J);                                                  \
     const float dy = py - a.y;                                                              \
     const float m1 = a.w * dy;                                                              \
     const float ev = fmaf(-b.x * dy, dy, b.y);                                              \
@@ -223,6 +235,7 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
       cr[p] = fmaf(c.x, w, cr[p]);                                                          \
       cg[p] = fmaf(c.y, w, cg[p]);                                                          \
       cb[p] = fmaf(c.z, w, cb[p]);                                                          \
+      if constexpr (MAPS) dd[p] = fmaf(dep, w, dd[p]);                                      \
       T[p] -= w;                                                                            \
     }                                                                                       \
   }
@@ -265,6 +278,34 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
   if (tid == 0 && k < nchunks) {
     for (int kk = k + 1; kk < nchunks && kk < k + FWD_STAGES; ++kk)
       gs_mbar_wait(&sm.full[kk % FWD_STAGES], (uint32_t)((kk / FWD_STAGES) & 1));
+  }
+  if constexpr (MAPS) {
+    // background behind the remaining transmittance; depth and alpha planes (PX floats = 16-byte aligned rows)
+    float av[FWD_PX];
+#pragma unroll
+    for (int p = 0; p < FWD_PX; ++p) {
+      cr[p] = fmaf(T[p], maps.bg_r, cr[p]);
+      cg[p] = fmaf(T[p], maps.bg_g, cg[p]);
+      cb[p] = fmaf(T[p], maps.bg_b, cb[p]);
+      av[p] = 1.f - T[p];
+    }
+    float4* od = reinterpret_cast<float4*>(maps.depth + (size_t)iy * wp + ix0);
+    float4* oa = reinterpret_cast<float4*>(maps.alpha + (size_t)iy * wp + ix0);
+#pragma unroll
+    for (int q = 0; q < FWD_PX / 4; ++q) {
+      od[q] = make_float4(dd[4 * q], dd[4 * q + 1], dd[4 * q + 2], dd[4 * q + 3]);
+      oa[q] = make_float4(av[4 * q], av[4 * q + 1], av[4 * q + 2], av[4 * q + 3]);
+    }
+    if (maps.depth_final) {
+#pragma unroll
+      for (int p = 0; p < FWD_PX; ++p) {
+        const int x = ix0 + p - crop.left, y = iy - crop.top;
+        if (x >= 0 && x < crop.width && y >= 0 && y < crop.height) {
+          maps.depth_final[(size_t)y * crop.width + x] = dd[p];
+          maps.alpha_final[(size_t)y * crop.width + x] = av[p];
+        }
+      }
+    }
   }
   // PX pixels x 3 channels = PX * 12 contiguous, 16-byte aligned bytes
   {
@@ -694,7 +735,7 @@ __global__ void __launch_bounds__(WSF_CONS + 32) blend_fwd_ws_kernel(const float
 // xor-shuffles combine the quarters, and each of the 4 lanes stores one 16-byte piece of the
 // instance's gradient record.  ~13 instructions per (thread, instance) instead of ~42 for the
 // recursive-halving shuffle network; fixed summation order => bit-deterministic.
-template <int PX, int STAGES_, int RQ_>
+template <int PX, int STAGES_, int RQ_, int PW_ = 6>
 struct Bwd2Cfg {
   static constexpr int NT = 256 / PX;                        // consumer threads (64 or 32)
   static constexpr int TPR = GS_TILE / PX;                   // threads per pixel row
@@ -702,27 +743,40 @@ struct Bwd2Cfg {
   static constexpr int R = NT / RQ;                          // instances per reduction round
   static constexpr int SQ = NT / RQ;                         // source threads per reducer ("part")
   static constexpr int ROWS = SQ / TPR;                      // pixel rows per reducer
-  // strides (floats) of the partial buffer [instance][part][source thread][6]: part stride = 32/RQ and
+  // floats per (source thread, instance): 6, or 8 for a maps frame - the 7th sum (and a pad) then sits in a
+  // [part][source thread][2] block behind the [part][source thread][6] one, so both store streams keep their stride
+  static constexpr int PW = PW_;
+  // strides (floats) of the partial buffer [instance][part][source thread][6 (+2)]: part stride = 32/RQ and
   // instance stride = 2 (mod 32) make the 8-byte loads of a half-warp (16 / RQ instances x RQ parts) hit
-  // 16 distinct bank pairs; the 8-byte stores of 16 consecutive source threads (stride 6) are conflict free
-  static constexpr int QS = (SQ * 6 + 31) / 32 * 32 + 32 / RQ;
+  // 16 distinct bank pairs; the 8-byte stores of 16 consecutive source threads (stride 6, resp. 2) are conflict free
+  static constexpr int QS = (SQ * PW + 31) / 32 * 32 + 32 / RQ;
   static constexpr int IS = RQ * QS + 2 - (RQ * QS) % 32 + ((RQ * QS) % 32 > 2 ? 32 : 0);
   static constexpr int STAGES = STAGES_;
 };
 
-template <int PX, int STAGES, int RQ, bool GATHER, int CH>
+template <int PX, int STAGES, int RQ, bool GATHER, int CH, int PW = 6>
 struct Bwd2Smem : std::conditional<GATHER, GatherRing<CH, STAGES, 4>, WsRing<STAGES>>::type {
-  float part[Bwd2Cfg<PX, STAGES, RQ>::R * Bwd2Cfg<PX, STAGES, RQ>::IS];
+  float part[Bwd2Cfg<PX, STAGES, RQ, PW>::R * Bwd2Cfg<PX, STAGES, RQ, PW>::IS];
   float pyt[GS_TILE];
   int valid[2];
 };
 
-// one instance x this thread's row of PX pixels: recompute alpha, analytic d/d alpha, six partial sums
+// Upstream gradients of the depth and alpha maps for a thread's row of PX pixels (MAPS only)
 template <int PX>
+struct MapsGrad {
+  float gd[PX], ga[PX];
+};
+
+// one instance x this thread's row of PX pixels: recompute alpha, analytic d/d alpha, six partial sums.
+// MAPS: depth and alpha act as two more channels with per-instance "colours" d_i and 1 (gc += gD d_i + gA), and a
+// 7th sum gD w (the gradient of the instance's depth) goes to dst_d.
+template <int PX, bool MAPS = false>
 __device__ __forceinline__ void bwd_row(const float4 a, const float2 b, const float4 c, const float (&px)[PX],
                                         const float py, float (&T)[PX], float (&Rr)[PX], const float (&gr)[PX],
-                                        const float (&gg)[PX], const float (&gb)[PX], float2* __restrict__ dst) {
-  float s0 = 0.f, sx = 0.f, sxx = 0.f, c0 = 0.f, c1 = 0.f, c2 = 0.f;
+                                        const float (&gg)[PX], const float (&gb)[PX], float2* __restrict__ dst,
+                                        const float dep = 0.f, const MapsGrad<PX>* mg = nullptr,
+                                        float2* __restrict__ dst_d = nullptr) {
+  float s0 = 0.f, sx = 0.f, sxx = 0.f, c0 = 0.f, c1 = 0.f, c2 = 0.f, cd = 0.f;
   const float dy = py - a.y;
   const float m1 = a.w * dy;
   const float ev = fmaf(-b.x * dy, dy, b.y);
@@ -733,7 +787,11 @@ __device__ __forceinline__ void bwd_row(const float4 a, const float2 b, const fl
     float alpha = gs_ex2(fmaf(-dx, eu, ev));                     // l2o - (ca dx^2 - cb dx dy + cc dy^2)
     alpha = (T[p] > GS_T_STOP) ? alpha : 0.f;                    // early stop (:578): no weight, no gradient
     const float w = alpha * T[p];
-    const float gc = fmaf(gr[p], c.x, fmaf(gg[p], c.y, gb[p] * c.z));
+    float gc = fmaf(gr[p], c.x, fmaf(gg[p], c.y, gb[p] * c.z));
+    if constexpr (MAPS) {
+      gc = fmaf(mg->gd[p], dep, gc + mg->ga[p]);
+      cd = fmaf(mg->gd[p], w, cd);
+    }
     Rr[p] = fmaf(-gc, w, Rr[p]);                                 // sum_c g_c (out_c - C_c^{<=i})
     const float rc = gs_rcp(1.0000001f - alpha);                 // 1/(1 - alpha + 1e-7)  (:721)
     const float dal = fmaf(T[p], gc, -Rr[p] * rc);               // d L / d alpha            (:710-722)
@@ -750,24 +808,30 @@ __device__ __forceinline__ void bwd_row(const float4 a, const float2 b, const fl
   dst[0] = make_float2(s0, sx);
   dst[1] = make_float2(sxx, c0);
   dst[2] = make_float2(c1, c2);
+  if constexpr (MAPS) dst_d[0] = make_float2(cd, 0.f);
 }
 
 // WS: dedicated producer warp (full / empty mbarrier ring); !WS: consumer thread 0 issues the copies at the
 // chunk boundaries (no extra warp holding registers).  UNR: instances per unrolled step of the first phase.
-template <int PX, bool WS, int UNR, int STAGES, int MINB, int RQ, bool GATHER, int CH>
+// MAPS (gather path only): gradients of the depth / alpha maps too; d/d depth_i goes to float 9 of the gradient row.
+// `maps` is the last parameter so that the other instantiations keep their parameter offsets (and their code).
+template <int PX, bool WS, int UNR, int STAGES, int MINB, int RQ, bool GATHER, int CH, bool MAPS = false>
 __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
     blend_bwd2_kernel(const float4* __restrict__ pA, const float2* __restrict__ pB, const float4* __restrict__ pC,
                       const GsRec* __restrict__ grec, const uint32_t* __restrict__ ids,
                       const uint32_t* __restrict__ goff, const int* __restrict__ tile_accum, int wp, int hp, int ntx, float fx, float fy,
                       const float* __restrict__ image, const float* __restrict__ grad_image,
                       float* __restrict__ grad_inst, int grad_is_final, GsCrop crop, uint32_t* __restrict__ row_epoch,
-                      uint32_t epoch, int* __restrict__ tile_neff_b) {
-  using Cfg = Bwd2Cfg<PX, STAGES, RQ>;
+                      uint32_t epoch, int* __restrict__ tile_neff_b, GsMapsBwd maps = GsMapsBwd{}) {
+  constexpr int PW = MAPS ? 8 : 6;
+  using Cfg = Bwd2Cfg<PX, STAGES, RQ, PW>;
   constexpr int NT = Cfg::NT, TPR = Cfg::TPR, R = Cfg::R, SQ = Cfg::SQ, QS = Cfg::QS, IS = Cfg::IS, ROWS = Cfg::ROWS;
   static_assert(IS % 2 == 0 && QS % 2 == 0 && IS % 32 == 2 && QS % 32 == 32 / RQ, "partial buffer strides");
   static_assert(!(WS && GATHER), "the gather path issues its copies from all consumer threads");
   static_assert(GATHER || CH == WS_CH, "the packed ring is sized for CH instances per stage");
-  using Smem = Bwd2Smem<PX, STAGES, RQ, GATHER, CH>;
+  static_assert(!MAPS || GATHER, "depth / alpha maps read the depth from the gathered records");
+  static_assert(PX % 4 == 0, "float4 rows of the image / map planes");
+  using Smem = Bwd2Smem<PX, STAGES, RQ, GATHER, CH, PW>;
   __shared__ __align__(16) Smem sm;
   const int tile = blockIdx.x;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -843,11 +907,46 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
       T[p] = 1.f;
     }
   }
+  MapsGrad<PX> mg;
+  if constexpr (MAPS) {
+    // the suffix sum starts at g . image + gD depth + gA alpha (the raw maps of the forward)
+    const size_t po = (size_t)iy * wp + ix0;          // PX floats = 16-byte aligned rows of the [Hp,Wp] planes
+    float dv[PX], av[PX];
+#pragma unroll
+    for (int q = 0; q < PX / 4; ++q) {
+      const float4 d4 = reinterpret_cast<const float4*>(maps.depth + po)[q];
+      const float4 a4 = reinterpret_cast<const float4*>(maps.alpha + po)[q];
+      dv[4 * q] = d4.x; dv[4 * q + 1] = d4.y; dv[4 * q + 2] = d4.z; dv[4 * q + 3] = d4.w;
+      av[4 * q] = a4.x; av[4 * q + 1] = a4.y; av[4 * q + 2] = a4.z; av[4 * q + 3] = a4.w;
+    }
+    if (!grad_is_final) {
+#pragma unroll
+      for (int q = 0; q < PX / 4; ++q) {
+        const float4 d4 = reinterpret_cast<const float4*>(maps.grad_depth + po)[q];
+        const float4 a4 = reinterpret_cast<const float4*>(maps.grad_alpha + po)[q];
+        mg.gd[4 * q] = d4.x; mg.gd[4 * q + 1] = d4.y; mg.gd[4 * q + 2] = d4.z; mg.gd[4 * q + 3] = d4.w;
+        mg.ga[4 * q] = a4.x; mg.ga[4 * q + 1] = a4.y; mg.ga[4 * q + 2] = a4.z; mg.ga[4 * q + 3] = a4.w;
+      }
+    } else {
+      // cropped [H,W] gradients: no clamp on the maps, nothing outside the crop
+#pragma unroll
+      for (int p = 0; p < PX; ++p) {
+        const int x = ix0 + p - crop.left, y = iy - crop.top;
+        const bool in = x >= 0 && x < crop.width && y >= 0 && y < crop.height;
+        mg.gd[p] = in ? maps.grad_depth[(size_t)y * crop.width + x] : 0.f;
+        mg.ga[p] = in ? maps.grad_alpha[(size_t)y * crop.width + x] : 0.f;
+      }
+    }
+#pragma unroll
+    for (int p = 0; p < PX; ++p) Rr[p] = fmaf(mg.gd[p], dv[p], fmaf(mg.ga[p], av[p], Rr[p]));
+  }
   // this thread's slot in the partial buffer: quarter tid / SQ, position tid % SQ
   float2* const my_part = reinterpret_cast<float2*>(sm.part + (tid / SQ) * QS + (tid % SQ) * 6);
+  float2* const my_part_d = reinterpret_cast<float2*>(sm.part + (tid / SQ) * QS + SQ * 6 + (tid % SQ) * 2);
   // second-phase role: instance ri of the round, quarter rq of the source threads
   const int ri = tid / RQ, rq = tid % RQ;
   const float2* const red_src = reinterpret_cast<const float2*>(sm.part + ri * IS + rq * QS);
+  const float2* const red_src_d = reinterpret_cast<const float2*>(sm.part + ri * IS + rq * QS + SQ * 6);
 
   int consumed = cnt;
   bool finished = false;
@@ -883,12 +982,14 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
         }
 #pragma unroll
         for (int u = 0; u < UNR; ++u)
-          bwd_row<PX>(sv.a(sub + j + u), sv.b(sub + j + u), sv.c(sub + j + u), px, py, T, Rr, gr, gg, gb,
-                      my_part + (j + u) * (IS / 2));
+          bwd_row<PX, MAPS>(sv.a(sub + j + u), sv.b(sub + j + u), sv.c(sub + j + u), px, py, T, Rr, gr, gg, gb,
+                            my_part + (j + u) * (IS / 2), MAPS ? sv.depth(sub + j + u) : 0.f, &mg,
+                            my_part_d + (j + u) * (IS / 2));
       }
       if (UNR > 1 && !wdead)
         for (; j < nr; ++j)
-          bwd_row<PX>(sv.a(sub + j), sv.b(sub + j), sv.c(sub + j), px, py, T, Rr, gr, gg, gb, my_part + j * (IS / 2));
+          bwd_row<PX, MAPS>(sv.a(sub + j), sv.b(sub + j), sv.c(sub + j), px, py, T, Rr, gr, gg, gb,
+                            my_part + j * (IS / 2), MAPS ? sv.depth(sub + j) : 0.f, &mg, my_part_d + j * (IS / 2));
       bool dead = true;
 #pragma unroll
       for (int p = 0; p < PX; ++p) dead = dead && !(T[p] > GS_T_STOP);
@@ -906,7 +1007,7 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
       }
       // ---- phase 2: 4 threads per instance, one quarter of the source threads (4 pixel rows) each
       {
-        float S0 = 0.f, Sx = 0.f, Sxx = 0.f, Sy = 0.f, Sxy = 0.f, Syy = 0.f, C0 = 0.f, C1 = 0.f, C2 = 0.f;
+        float S0 = 0.f, Sx = 0.f, Sxx = 0.f, Sy = 0.f, Sxy = 0.f, Syy = 0.f, C0 = 0.f, C1 = 0.f, C2 = 0.f, Cd = 0.f;
         const bool act = ri < nr;
         float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
         float2 b = make_float2(0.f, 0.f);
@@ -935,6 +1036,12 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
             Sy = fmaf(dyr, u0.x, Sy);
             Sxy = fmaf(dyr, u0.y, Sxy);
             Syy = fmaf(dyr * dyr, u0.x, Syy);
+            if constexpr (MAPS) {
+              float ud = red_src_d[r * TPR].x;
+#pragma unroll
+              for (int t = 1; t < TPR; ++t) ud += red_src_d[r * TPR + t].x;
+              Cd += ud;
+            }
           }
         }
 #define GS_RED4(V)                                   \
@@ -942,18 +1049,19 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
   V += __shfl_xor_sync(0xffffffffu, V, 2);           \
   if (RQ == 8) V += __shfl_xor_sync(0xffffffffu, V, 4);
         GS_RED4(S0) GS_RED4(Sx) GS_RED4(Sxx) GS_RED4(Sy) GS_RED4(Sxy) GS_RED4(Syy) GS_RED4(C0) GS_RED4(C1) GS_RED4(C2)
+        if constexpr (MAPS) { GS_RED4(Cd) }
 #undef GS_RED4
         if (act) {
           const uint32_t slot = sv.slot(sub + ri, tx, ty);
           float4* out = reinterpret_cast<float4*>(grad_inst + (size_t)slot * GS_GREC);
-          // d/dx, d/dy, d/dca, d/dcb  |  d/dcc, d/dl2o, d/dr, d/dg  |  d/db
+          // d/dx, d/dy, d/dca, d/dcb  |  d/dcc, d/dl2o, d/dr, d/dg  |  d/db (, d/ddepth: maps frames)
           if (rq == 0)
             out[0] = make_float4(GS_LN2 * (2.f * a.z * Sx - a.w * Sy), GS_LN2 * (2.f * b.x * Sy - a.w * Sx),
                                  -GS_LN2 * Sxx, GS_LN2 * Sxy);
           else if (rq == 1)
             out[1] = make_float4(-GS_LN2 * Syy, GS_LN2 * S0, C0, C1);
           else if (rq == 2)
-            out[2] = make_float4(C2, 0.f, 0.f, 0.f);
+            out[2] = make_float4(C2, MAPS ? Cd : 0.f, 0.f, 0.f);
           else if (rq == 3 && row_epoch)
             row_epoch[slot] = epoch;               // marks the row as written in this frame
         }
@@ -1233,6 +1341,35 @@ cudaError_t gs_launch_blend_bwd(const float4* pA, const float2* pB, const float4
   else if (ch == 128) GS_BWD_LAUNCH(2, 128);
   else GS_BWD_LAUNCH(2, 64);
 #undef GS_BWD_LAUNCH
+  return cudaGetLastError();
+}
+
+// Maps frames always run the shipped gather configurations (forward: 128-instance chunks, 4 pixels per thread;
+// backward: 8 pixels per thread, 4-instance unroll, 3 stages, MINB 10, 4 reducers, 32-instance chunks).
+cudaError_t gs_launch_blend_fwd_maps(const GsRec* grec, const uint32_t* ids, const int* tile_accum, const GsFrameGeom& g,
+                                     float* image, int* tile_neff, float* final_img, const GsCrop& crop,
+                                     const GsMapsFwd& maps, cudaStream_t st) {
+  // grec / ids may be null: a frame without tile instances (no Gaussian, or none visible, on a context that never
+  // had one) never reads them - every tile is empty and renders the background with depth = alpha = 0
+  if (!maps.depth || !maps.alpha || (final_img != nullptr) != (maps.depth_final != nullptr) ||
+      (maps.depth_final != nullptr) != (maps.alpha_final != nullptr))
+    return cudaErrorInvalidValue;
+  blend_fwd_kernel<128, 4, true, true><<<g.n_tiles, 64, 0, st>>>(nullptr, nullptr, nullptr, grec, ids, tile_accum, g.wp,
+                                                                 g.hp, g.ntx, g.fx, g.fy, image, tile_neff, final_img,
+                                                                 crop, maps);
+  return cudaGetLastError();
+}
+
+cudaError_t gs_launch_blend_bwd_maps(const GsRec* grec, const uint32_t* ids, const uint32_t* goff, const int* tile_accum,
+                                     const GsFrameGeom& g, const float* image, const float* grad_image, float* grad_inst,
+                                     int grad_is_final, const GsCrop& crop, uint32_t* row_epoch, uint32_t epoch,
+                                     int* tile_neff_b, const GsMapsBwd& maps, cudaStream_t st) {
+  // only launched for frames with tile instances (an empty frame has no blend backward), so the records exist
+  if (!grec || !ids || !goff || !row_epoch || !maps.depth || !maps.alpha || !maps.grad_depth || !maps.grad_alpha)
+    return cudaErrorInvalidValue;
+  blend_bwd2_kernel<8, false, 4, 3, 10, 4, true, 32, true><<<g.n_tiles, 32, 0, st>>>(
+      nullptr, nullptr, nullptr, grec, ids, goff, tile_accum, g.wp, g.hp, g.ntx, g.fx, g.fy, image, grad_image,
+      grad_inst, grad_is_final, crop, row_epoch, epoch, tile_neff_b, maps);
   return cudaGetLastError();
 }
 

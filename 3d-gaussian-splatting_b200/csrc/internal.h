@@ -22,6 +22,25 @@ struct GsCrop {
   int left, top, width, height;
 };
 
+// Depth / alpha maps and a background colour (gs_render_forward_maps; RGB gather path only).  Per pixel, over the
+// instances the colour blend uses: image += T_end * bg, depth = sum w_i d_i (d_i = |p_c|, GsRec.c.y), alpha = 1 - T_end.
+// Forward: raw padded planes [Hp,Wp]; the cropped [H,W] planes (no clamp) when the final layout is requested.
+struct GsMapsFwd {
+  float* depth;
+  float* alpha;
+  float* depth_final;           // nullable (with final_img == nullptr)
+  float* alpha_final;
+  float bg_r, bg_g, bg_b;
+};
+// Backward: the forward's raw planes and the gradients of the depth / alpha maps (padded, or cropped [H,W] when
+// grad_is_final; zero outside the crop, no clamp mask)
+struct GsMapsBwd {
+  const float* depth;
+  const float* alpha;
+  const float* grad_depth;
+  const float* grad_alpha;
+};
+
 // world-space ray setup for per-pixel SH (reference splatter.py:305-321), DEVICE pointers to 3 floats each
 struct GsRayPtrs {
   const float *rays_o, *lefttop, *dx, *dy;
@@ -96,7 +115,8 @@ cudaError_t gs_launch_fused_project_bwd(const float* pos, const float* rgb, cons
                                         float near_plane, float half_w, float half_h, const uint32_t* offsets_g,
                                         const uint32_t* count, const float* grad_inst, const uint32_t* row_epoch, uint32_t epoch,
                                         float* g_pos, float* g_rgb, float* g_opa,
-                                        float* g_quat, float* g_scale, const GsGradPush& push, cudaStream_t st);
+                                        float* g_quat, float* g_scale, const GsGradPush& push, cudaStream_t st,
+                                        bool depth_grad = false /*maps frame: chain float 9 of the rows to pos*/);
 
 // ---- binning.cu ------------------------------------------------------------------------
 cudaError_t gs_launch_emit_keys(const GsRec* rec, const uint32_t* perm, const uint32_t* offsets_sorted, int n, int ntx,
@@ -127,3 +147,13 @@ cudaError_t gs_launch_blend_bwd(const float4* pA, const float2* pB, const float4
                                 int grad_is_final, const GsCrop& crop, uint32_t* row_epoch /*nullable (packed only)*/,
                                 uint32_t epoch, int* tile_neff_b /*nullable: instances the backward consumed per tile*/,
                                 cudaStream_t st);
+
+// Maps frame (gather path, fixed configuration: the gs_tune knobs do not apply).  The backward additionally writes
+// d/d depth_i = sum g_D w into float 9 of every gradient row.
+cudaError_t gs_launch_blend_fwd_maps(const GsRec* grec, const uint32_t* ids, const int* tile_accum, const GsFrameGeom& g,
+                                     float* image, int* tile_neff, float* final_img, const GsCrop& crop,
+                                     const GsMapsFwd& maps, cudaStream_t st);
+cudaError_t gs_launch_blend_bwd_maps(const GsRec* grec, const uint32_t* ids, const uint32_t* goff, const int* tile_accum,
+                                     const GsFrameGeom& g, const float* image, const float* grad_image, float* grad_inst,
+                                     int grad_is_final, const GsCrop& crop, uint32_t* row_epoch, uint32_t epoch,
+                                     int* tile_neff_b, const GsMapsBwd& maps, cudaStream_t st);

@@ -140,7 +140,9 @@ __device__ __forceinline__ void push_store(const GsGradPush& P, float* local, co
   }
 }
 
-template <int D, int GW, int W>
+// DEPTH (maps frames, D == 3): float 9 of the rows is d/d|p_c| and is chained to pos; otherwise the depth is only a
+// sort key.
+template <int D, int GW, int W, bool DEPTH = false>
 __global__ void __launch_bounds__(kBlock) fused_project_bwd_kernel(
     const float* __restrict__ pos, const float* __restrict__ rgb, const float* __restrict__ opa,
     const float* __restrict__ quat, const float* __restrict__ scale, int n, int scale_act, GsCam cam,
@@ -199,7 +201,8 @@ __global__ void __launch_bounds__(kBlock) fused_project_bwd_kernel(
     gcov[1] = acc[3] * sc + gsc * kk * o.c;                   // d det/db = -c
     gcov[2] = acc[3] * sc + gsc * kk * o.b;                   // d det/dc = -b
     gcov[3] = acc[2] * sc - gsc * kk * o.a;                   // d det/dd =  a
-    float gxyd[3] = {acc[0], acc[1], 0.f};                    // depth is only a sort key
+    static_assert(!DEPTH || D == 3, "the depth gradient has a row slot in the RGB layout only");
+    float gxyd[3] = {acc[0], acc[1], DEPTH ? acc[9] : 0.f};   // depth: sort key, + map gradient in maps frames
     float gq[4], gsv[3];
     gs_project_backward(cam, p, q, s, gxyd, gcov, gp, gq, gsv);
     // quat normalisation backward: q = r/|r|
@@ -435,8 +438,16 @@ cudaError_t gs_launch_fused_project_bwd(const float* pos, const float* rgb, cons
                                         float near_plane, float half_w, float half_h, const uint32_t* offsets_g,
                                         const uint32_t* count, const float* grad_inst, const uint32_t* row_epoch, uint32_t epoch,
                                         float* g_pos, float* g_rgb, float* g_opa,
-                                        float* g_quat, float* g_scale, const GsGradPush& push, cudaStream_t st) {
+                                        float* g_quat, float* g_scale, const GsGradPush& push, cudaStream_t st,
+                                        bool depth_grad) {
   if (n == 0) return cudaSuccess;
+  if (depth_grad) {
+    if (d != 3 || push.world != 0) return cudaErrorInvalidValue;
+    fused_project_bwd_kernel<3, GS_GREC, 0, true><<<grid_for(n), kBlock, 0, st>>>(
+        pos, rgb, opa, quat, scale, n, scale_act, cam, near_plane, half_w, half_h, offsets_g, count, grad_inst, row_epoch,
+        epoch, g_pos, g_rgb, g_opa, g_quat, g_scale, push);
+    return cudaGetLastError();
+  }
 #define GS_LAUNCH_PBWD(D, GW, W)                                                                                    \
   fused_project_bwd_kernel<D, GW, W><<<grid_for(n), kBlock, 0, st>>>(pos, rgb, opa, quat, scale, n, scale_act, cam, \
                                                                      near_plane, half_w, half_h, offsets_g, count, \

@@ -53,8 +53,7 @@ GsTuning& gs_tuning() {
                        tune_env("GS_TUNE_GATHER", 1),      tune_env("GS_TUNE_SH_TC", 3)};
   return t;
 }
-extern "C" int gs_tune(const char* name, int value) {
-  if (!name) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_tune: null name");
+static int* tune_knob(const char* name) {
   GsTuning& t = gs_tuning();
   struct { const char* k; int* v; } tab[] = {{"fwd_kernel", &t.fwd_kernel}, {"fwd_ch", &t.fwd_ch},
                                              {"bwd_kernel", &t.bwd_kernel}, {"bwd_px", &t.bwd_px},
@@ -64,11 +63,22 @@ extern "C" int gs_tune(const char* name, int value) {
                                              {"gather", &t.gather},         {"bwd_ch", &t.bwd_ch},
                                              {"strict", &t.strict},         {"sh_tc", &t.sh_tc}};
   for (auto& e : tab)
-    if (!strcmp(e.k, name)) {
-      *e.v = value;
-      return 0;
-    }
-  return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_tune: unknown knob");
+    if (!strcmp(e.k, name)) return e.v;
+  return nullptr;
+}
+extern "C" int gs_tune(const char* name, int value) {
+  if (!name) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_tune: null name");
+  int* v = tune_knob(name);
+  if (!v) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_tune: unknown knob");
+  *v = value;
+  return 0;
+}
+extern "C" int gs_tune_get(const char* name, int* value) {
+  if (!name || !value) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_tune_get: null argument");
+  const int* v = tune_knob(name);
+  if (!v) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_tune_get: unknown knob");
+  *value = *v;
+  return 0;
 }
 
 #include <atomic>
@@ -141,6 +151,7 @@ struct gs_ctx {
   cudaEvent_t ev_m = nullptr;             // marks the completion of the M read-back
   // state of the last forward
   bool have_forward = false, have_backward = false, gather = false;
+  bool maps = false;                      // the last forward also wrote depth / alpha maps (gs_render_forward_maps)
   int n = 0, d = 3, scale_act = 0;
   long long m = 0;
   GsCam cam{};
@@ -218,9 +229,25 @@ static int ceil_log2(unsigned v) {
   return b;
 }
 
+// a maps frame needs the RGB gather path and one GPU's gradient layout; returns 0 or the refusal
+static int check_maps_supported(const gs_ctx* c, int d, const char* fn) {
+  char msg[200];
+  const char* why = nullptr;
+  if (d != 3)
+    why = "depth / alpha maps need RGB colour (d == 3); SH colour is not supported";
+  else if (gs_tuning().gather == 0)
+    why = "depth / alpha maps need the gather path (gs_tune(\"gather\", 0) is set)";
+  else if (c->push.world != 0)
+    why = "depth / alpha maps do not support the data-parallel gradient push (gs_ctx_set_grad_push is active)";
+  if (!why) return 0;
+  snprintf(msg, sizeof(msg), "%s: %s", fn, why);
+  return gs_set_error_msg(GS_ERR_UNSUPPORTED, msg);
+}
+
 static int render_forward_impl(gs_ctx* c, const float* pos, const float* rgb, const float* opa, const float* quat,
                                const float* scale, int n, int d, int scale_activation, const gs_camera* cam,
-                               float* image, float* final_img, int64_t* culling_mask, gs_stream_t stream) {
+                               float* image, float* final_img, int64_t* culling_mask, gs_stream_t stream,
+                               const GsMapsFwd* maps = nullptr) {
   if (!c || !cam || n < 0) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_render_forward: bad arguments");
   if (d != 3 && gs_sh_basis_count(d) == 0)
     return gs_set_error_msg(GS_ERR_UNSUPPORTED, "gs_render_forward: colour width must be 3 (RGB), 27 (SH deg 2) or 48 (SH deg 3)");
@@ -230,10 +257,13 @@ static int render_forward_impl(gs_ctx* c, const float* pos, const float* rgb, co
     return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_render_forward: tile_thresh must be in (0, 1)");
   if (!image || (n > 0 && (!pos || !rgb || !opa || !quat || !scale)))
     return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_render_forward: null tensor pointer");
+  if (maps)
+    if (int rc = check_maps_supported(c, d, "gs_render_forward_maps")) return rc;
   if (int rc = gs_check_device(c->device, "gs_render_forward")) return rc;
   g_cur_alloc = &c->allocator;
   cudaStream_t st = (cudaStream_t)stream;
   c->have_forward = false;
+  c->maps = false;
   c->have_backward = false;
 
   GsFrameGeom g{};
@@ -423,7 +453,10 @@ static int render_forward_impl(gs_ctx* c, const float* pos, const float* rgb, co
   // 6. blend (+ optional fused clamp & centre crop, splatter.py:652-653 / :267-272)
   GsCrop crop{(g.wp - g.width) / 2, (g.hp - g.height) / 2, g.width, g.height};
   gs_mark(c, 5, st);
-  if (d == 3) {
+  if (maps) {
+    GS_CUDA_TRY(gs_launch_blend_fwd_maps(c->rec.as<GsRec>(), c->vals_out.as<uint32_t>(), c->tile_accum.as<int>(), g, image,
+                                         c->tile_neff.as<int>(), final_img, crop, *maps, st));
+  } else if (d == 3) {
     GS_CUDA_TRY(gs_launch_blend_fwd(c->pA.as<float4>(), c->pB.as<float2>(), c->pC.as<float4>(),
                                     gather ? c->rec.as<GsRec>() : nullptr, c->vals_out.as<uint32_t>(),
                                     c->tile_accum.as<int>(), g, image, c->tile_neff.as<int>(), final_img, crop, st));
@@ -441,6 +474,7 @@ static int render_forward_impl(gs_ctx* c, const float* pos, const float* rgb, co
   c->ev_fwd_valid = c->timing && c->ev_ok;
 
   c->have_forward = true;
+  c->maps = maps != nullptr;
   c->gather = gather;
   c->n = n;
   c->d = d;
@@ -474,9 +508,17 @@ extern "C" int gs_render_forward_final(gs_ctx* c, const float* pos, const float*
 static int render_backward_impl(gs_ctx* c, const float* pos, const float* rgb, const float* opa, const float* quat,
                                 const float* scale, const float* image, const float* grad_image, int grad_is_final,
                                 float* grad_pos, float* grad_rgb, float* grad_opa, float* grad_quat,
-                                float* grad_scale, gs_stream_t stream) {
+                                float* grad_scale, gs_stream_t stream, const GsMapsBwd* maps = nullptr) {
   if (!c) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_render_backward: null ctx");
   if (!c->have_forward) return gs_set_error_msg(GS_ERR_NO_FORWARD, "gs_render_backward: no forward on this ctx");
+  if (maps) {
+    if (!c->maps)
+      return gs_set_error_msg(GS_ERR_NO_FORWARD,
+                              "gs_render_backward_maps: the last forward on this ctx was not gs_render_forward_maps");
+    if (int rc = check_maps_supported(c, c->d, "gs_render_backward_maps")) return rc;
+    if (!maps->depth || !maps->alpha || !maps->grad_depth || !maps->grad_alpha)
+      return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_render_backward_maps: null map pointer");
+  }
   if (!image || !grad_image || !grad_pos || !grad_rgb || !grad_opa || !grad_quat || !grad_scale ||
       (c->n > 0 && (!pos || !rgb || !opa || !quat || !scale)))
     return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_render_backward: null tensor pointer");
@@ -502,7 +544,12 @@ static int render_backward_impl(gs_ctx* c, const float* pos, const float* rgb, c
   GsCrop crop{(c->geom.wp - c->geom.width) / 2, (c->geom.hp - c->geom.height) / 2, c->geom.width, c->geom.height};
   gs_mark(c, 7, st);
   if (c->m > 0) {
-    if (d == 3) {
+    if (maps) {
+      GS_CUDA_TRY(gs_launch_blend_bwd_maps(c->rec.as<GsRec>(), c->vals_out.as<uint32_t>(), c->offsets_g.as<uint32_t>(),
+                                           c->tile_accum.as<int>(), c->geom, image, grad_image, c->grad_inst.as<float>(),
+                                           grad_is_final, crop, c->row_epoch.as<uint32_t>(), c->epoch,
+                                           c->tile_neff_b.as<int>(), *maps, st));
+    } else if (d == 3) {
       GS_CUDA_TRY(gs_launch_blend_bwd(c->pA.as<float4>(), c->pB.as<float2>(), c->pC.as<float4>(),
                                       c->gather ? c->rec.as<GsRec>() : nullptr, c->vals_out.as<uint32_t>(),
                                       c->offsets_g.as<uint32_t>(), c->tile_accum.as<int>(), c->geom, image, grad_image,
@@ -539,7 +586,8 @@ static int render_backward_impl(gs_ctx* c, const float* pos, const float* rgb, c
   GS_CUDA_TRY(gs_launch_fused_project_bwd(pos, rgb, opa, quat, scale, c->n, d, c->scale_act, c->cam, c->near_plane,
                                           c->half_w, c->half_h, c->offsets_g.as<uint32_t>(), c->count.as<uint32_t>(),
                                           c->grad_inst.as<float>(), c->row_epoch.as<uint32_t>(), c->epoch,
-                                          grad_pos, grad_rgb, grad_opa, grad_quat, grad_scale, c->push, st));
+                                          grad_pos, grad_rgb, grad_opa, grad_quat, grad_scale, c->push, st,
+                                          maps != nullptr));
   if (c->n > 0) gs_count_launch();
   gs_mark(c, 9, st);
   c->ev_bwd_valid = c->timing && c->ev_ok;
@@ -560,6 +608,39 @@ extern "C" int gs_render_backward_final(gs_ctx* c, const float* pos, const float
                                         float* grad_quat, float* grad_scale, gs_stream_t stream) {
   return render_backward_impl(c, pos, rgb, opa, quat, scale, image_raw_padded, grad_final, 1, grad_pos, grad_rgb,
                               grad_opa, grad_quat, grad_scale, stream);
+}
+
+extern "C" int gs_render_forward_maps(gs_ctx* c, const float* pos, const float* rgb, const float* opa, const float* quat,
+                                      const float* scale, int n, int d, int scale_activation, const gs_camera* cam,
+                                      const float* background_host, float* image_raw_padded, float* depth_raw_padded,
+                                      float* alpha_raw_padded, float* image_final, float* depth_final, float* alpha_final,
+                                      int64_t* culling_mask, gs_stream_t stream) {
+  if (!c) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_render_forward_maps: null ctx");
+  if (!depth_raw_padded || !alpha_raw_padded)
+    return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_render_forward_maps: null depth / alpha plane");
+  const bool fin = image_final != nullptr;
+  if ((depth_final != nullptr) != fin || (alpha_final != nullptr) != fin)
+    return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_render_forward_maps: the three final outputs must be all NULL or all set");
+  GsMapsFwd maps{depth_raw_padded, alpha_raw_padded, depth_final, alpha_final, 0.f, 0.f, 0.f};
+  if (background_host) {
+    maps.bg_r = background_host[0];
+    maps.bg_g = background_host[1];
+    maps.bg_b = background_host[2];
+  }
+  return render_forward_impl(c, pos, rgb, opa, quat, scale, n, d, scale_activation, cam, image_raw_padded, image_final,
+                             culling_mask, stream, &maps);
+}
+
+extern "C" int gs_render_backward_maps(gs_ctx* c, const float* pos, const float* rgb, const float* opa,
+                                       const float* quat, const float* scale, const float* image_raw_padded,
+                                       const float* depth_raw_padded, const float* alpha_raw_padded,
+                                       const float* grad_image, const float* grad_depth, const float* grad_alpha,
+                                       int grad_is_final, float* grad_pos, float* grad_rgb, float* grad_opa,
+                                       float* grad_quat, float* grad_scale, gs_stream_t stream) {
+  if (!c) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_render_backward_maps: null ctx");
+  GsMapsBwd maps{depth_raw_padded, alpha_raw_padded, grad_depth, grad_alpha};
+  return render_backward_impl(c, pos, rgb, opa, quat, scale, image_raw_padded, grad_image, grad_is_final ? 1 : 0,
+                              grad_pos, grad_rgb, grad_opa, grad_quat, grad_scale, stream, &maps);
 }
 
 extern "C" int gs_ctx_set_grad_push(gs_ctx* c, const gs_grad_push* p) {

@@ -5,7 +5,8 @@ conventions as reference renderer.py (`draw` :89, `trunc_exp` :102,
 `world2camera_func` :119, `global_culling` :158), so code written against the
 reference keeps working; underneath, every op calls the sm_100a kernels of
 libgs_b200 through the `gaussian` extension in this directory.  Additive:
-`render_frame`, one autograd node for the whole frame (fused path).
+`render_frame`, one autograd node for the whole frame (fused path), and `render_frame_maps`,
+the same frame with depth / alpha maps and a background colour.
 
 The product path never falls back to PyTorch/CPU math: importing this module
 without the built extension raises.
@@ -246,3 +247,46 @@ class _RenderFrameFinal(torch.autograd.Function):
 
 
 render_frame_final = _RenderFrameFinal.apply
+
+
+class _RenderFrameMaps(torch.autograd.Function):
+    """The frame of `render_frame` / `render_frame_final` plus a depth map (sum_i w_i |p_c,i|, not normalised), an
+    alpha map (1 - T_end) and a constant background colour (image += T_end * bg), all from the blend kernels in one
+    pass.  final=True: crop(clamp(image)) [H,W,3], crop(depth), crop(alpha) [H,W] (maps not clamped); else the
+    padded raw planes.  RGB colour only; the background gets no gradient."""
+
+    @staticmethod
+    def forward(ctx, rctx, pos, rgb, opa, quat, scale, width, height, focal_x, focal_y, rot, tran,
+                near, tile_thresh, scale_activation, background, final):
+        pos, rgb, opa, quat, scale = (_f32(t.detach()) for t in (pos, rgb, opa, quat, scale))
+        image, depth, alpha, raw, draw_, araw, mask = rctx.forward_maps(
+            pos, rgb, opa, quat, scale, int(width), int(height), float(focal_x), float(focal_y), rot.detach().cpu(),
+            tran.detach().cpu(), float(near), float(tile_thresh), SCALE_ACTIVATIONS[scale_activation], background,
+            bool(final))
+        ctx.rctx = rctx
+        ctx.frame = rctx.frame_id()
+        ctx.final = bool(final)
+        ctx.save_for_backward(pos, rgb, opa, quat, scale, raw, draw_, araw)
+        ctx.mark_non_differentiable(mask)
+        return image, depth, alpha, mask
+
+    @staticmethod
+    def backward(ctx, grad_image, grad_depth, grad_alpha, _grad_mask):
+        # autograd hands zeros for an output that received no gradient (materialised grads)
+        pos, rgb, opa, quat, scale, raw, draw_, araw = ctx.saved_tensors
+        outs, push = _flat_grads((pos, rgb, opa, quat, scale))
+        _apply_push(ctx.rctx, push)
+        ctx.rctx.backward_maps_into(pos, rgb, opa, quat, scale, raw, draw_, araw, _f32(grad_image), _f32(grad_depth),
+                                    _f32(grad_alpha), ctx.final, *outs, ctx.frame)
+        return (None, outs[0], outs[1], outs[2], outs[3], outs[4]) + (None,) * 11
+
+
+def render_frame_maps(rctx, pos, rgb, opa, quat, scale, width, height, focal_x, focal_y, rot, tran, near,
+                      tile_thresh, scale_activation, background=None, final=True):
+    """One autograd node: raw parameters -> (image, depth, alpha, culling_mask).  `background`: None (black) or
+    three floats.  A None gradient for any of the three images counts as zeros.  See `_RenderFrameMaps`."""
+    bg = None if background is None else [float(x) for x in background]
+    if bg is not None and len(bg) != 3:
+        raise ValueError("background must have 3 values (r, g, b)")
+    return _RenderFrameMaps.apply(rctx, pos, rgb, opa, quat, scale, width, height, focal_x, focal_y, rot, tran, near,
+                                  tile_thresh, scale_activation, bg, final)

@@ -9,7 +9,8 @@ splatter.py:324-345) and the surface train.py / visergui.py touch (train.py:57-6
 `ground_truth`, `imgs`, `culling_mask` (int64), `n_tile_gaussians`, `n_gaussians`, `device`,
 `scale_activation`, `set_camera`, `switch_resolution`.  Additionally
 `Splatter.from_tensors(gaussians, views, ...)` builds a scene without COLMAP (synthetic
-benchmarks / tests).
+benchmarks / tests) and `render_maps(...)` returns depth and alpha maps with the image, over an
+optional background colour.
 
 The per-frame work of reference `project_and_culling` + `render` (:513-634: 4 boolean-mask
 compactions, the dense [T, N/20] list, cumsum, two 4-tensor gathers, fp32-key sort, >= 7 host
@@ -27,7 +28,7 @@ import torch
 import torch.nn as nn
 
 import gaussian
-from renderer import render_frame, render_frame_final
+from renderer import render_frame, render_frame_final, render_frame_maps
 
 EPS = 1e-4
 SH_C0 = 0.28209479177387814
@@ -282,6 +283,22 @@ class Splatter(nn.Module):
         self.n_gaussians = g.pos.shape[0]
         self.n_tile_gaussians = self._rctx.last_instances()         # train.py:198 reads it every step
         return image
+
+    def render_maps(self, camera_id=None, extrinsics=None, intrinsics=None, background=None):
+        """Like `forward`, plus the depth and alpha maps, over an optional constant background colour
+        (three floats; None = black, i.e. `forward`'s image).  Returns (image [H,W,3] clamped to [0,1],
+        depth [H,W] = sum_i w_i |p_c,i| (not normalised: expected depth = depth / alpha), alpha [H,W] =
+        1 - final transmittance), all differentiable; the maps are not clamped.  RGB colour only."""
+        self.set_camera(camera_id, extrinsics, intrinsics)
+        g, v = self.gaussian_3ds, self.current_view
+        image, depth, alpha, mask = render_frame_maps(self._rctx, g.pos, g.rgb, g.opa, g.quat, g.scale, v["width"],
+                                                      v["height"], v["focal_x"], v["focal_y"], v["rot"], v["tran"],
+                                                      self.near, self.tile_culling_prob_thresh, self.scale_activation,
+                                                      background=background, final=True)
+        self.culling_mask = mask
+        self.n_gaussians = g.pos.shape[0]
+        self.n_tile_gaussians = self._rctx.last_instances()
+        return image, depth, alpha
 
     def forward_unfused_post(self, camera_id=None, extrinsics=None, intrinsics=None):
         """Same image through the padded raw render + torch clamp/crop (kept for cross-checks)."""

@@ -38,6 +38,8 @@ const char* gs_last_error(void);
  * (see csrc/internal.h GsTuning).  An unsupported combination makes the next backward fail with
  * cudaErrorInvalidValue.  Process-wide, not thread-safe. */
 int gs_tune(const char* name, int value);
+/* New: current value of a gs_tune knob (e.g. to restore it after an experiment). */
+int gs_tune_get(const char* name, int* value);
 /* Number of kernels of THIS library launched by the process so far (library kernels such as CUB's are not
  * counted); bench.py reports the difference over its timed region as `gpu_launches`. */
 unsigned long long gs_kernel_launches(void);
@@ -184,6 +186,40 @@ int gs_render_backward_final(gs_ctx* ctx, const float* pos, const float* rgb, co
                              const float* quat, const float* scale, const float* image_raw_padded,
                              const float* grad_final, float* grad_pos, float* grad_rgb, float* grad_opa,
                              float* grad_quat, float* grad_scale, gs_stream_t stream);
+
+/* New (an extension, not a replacement of a reference function; the reference composites colour on black only):
+ * the frame of gs_render_forward[_final] plus a depth map, an alpha map and a background colour.
+ * For a pixel, over exactly the instances (and the early stop) of the colour blend, w_i = alpha_i T_i:
+ *   image = sum w_i c_i + T_end * background     (background_host: 3 host floats; NULL = black = gs_render_forward)
+ *   depth = sum w_i d_i,  d_i = |R p_i + t|       (the depth of global_culling's res_pos[:,2] and of the sort key;
+ *                                                  accumulated, not normalised: expected depth = depth / alpha)
+ *   alpha = 1 - T_end
+ * Writes image_raw_padded[Hp,Wp,3] (un-clamped), depth_raw_padded[Hp,Wp], alpha_raw_padded[Hp,Wp] and, when the
+ * three final pointers are set (all NULL or all set), image_final[height,width,3] = crop(clamp(image, 0, 1)),
+ * depth_final / alpha_final[height,width] = crop(.) with NO clamp.  Same launches and one host synchronisation,
+ * like gs_render_forward.  GS_ERR_UNSUPPORTED (reason in gs_last_error) for d != 3 (SH colour), with
+ * gs_tune("gather", 0), and while a gs_ctx_set_grad_push configuration is active.  The A/B tuning knobs of the
+ * blend kernels do not apply: a maps frame always runs the shipped gather configuration. */
+int gs_render_forward_maps(gs_ctx* ctx, const float* pos, const float* rgb, const float* opa,
+                           const float* quat, const float* scale, int n, int d, int scale_activation,
+                           const gs_camera* cam_host, const float* background_host,
+                           float* image_raw_padded, float* depth_raw_padded, float* alpha_raw_padded,
+                           float* image_final, float* depth_final, float* alpha_final,
+                           int64_t* culling_mask, gs_stream_t stream);
+/* New.  Backward of the most recent gs_render_forward_maps on ctx: the gradient of
+ * <grad_image, image> + <grad_depth, depth> + <grad_alpha, alpha> wrt the five RAW parameters (overwrites all n rows,
+ * like gs_render_backward).  The raw planes are the forward's outputs.  grad_is_final = 0: padded gradients
+ * ([Hp,Wp,3], [Hp,Wp], [Hp,Wp]); 1: gradients of the final outputs ([height,width,3], [height,width] x 2; the image
+ * clamp passes gradient where 0 <= raw <= 1, the maps have no clamp, the padding gets none).  Pass zero-filled
+ * planes for outputs without a gradient.  pos receives the direct depth term through d_i; the background is a
+ * constant (no gradient).  GS_ERR_NO_FORWARD if the last forward on ctx was not a maps forward; GS_ERR_UNSUPPORTED
+ * as for the forward.  No synchronisation. */
+int gs_render_backward_maps(gs_ctx* ctx, const float* pos, const float* rgb, const float* opa,
+                            const float* quat, const float* scale, const float* image_raw_padded,
+                            const float* depth_raw_padded, const float* alpha_raw_padded,
+                            const float* grad_image, const float* grad_depth, const float* grad_alpha,
+                            int grad_is_final, float* grad_pos, float* grad_rgb, float* grad_opa,
+                            float* grad_quat, float* grad_scale, gs_stream_t stream);
 
 /* Per-stage device timing with CUDA events recorded on the frame's stream (off by default).
  * gs_frame_stage_ms fills out[GS_N_STAGES] with the milliseconds of the last frame's stages:
