@@ -323,6 +323,20 @@ struct RenderContext {
   }
   void clear_grad_push() { check_rc(gs_ctx_set_grad_push(ctx, nullptr), "gs_ctx_set_grad_push"); }
 
+  // camera pose gradient (gs_ctx_set_camera_grad): every backward on this context also overwrites grad_cam[12] =
+  // (d/d rot row-major, d/d tran) while it is set; None clears it.  The tensor must outlive its use.
+  void set_camera_grad(c10::optional<torch::Tensor> grad_cam) {
+    float* p = nullptr;
+    if (grad_cam) {
+      const torch::Tensor& g = *grad_cam;
+      GS_CHECK_F32(g);
+      TORCH_CHECK(g.numel() == 12, "set_camera_grad: grad_cam must have 12 elements (9 rot + 3 tran)");
+      TORCH_CHECK(g.device().index() == device, "set_camera_grad: grad_cam is on another device than the RenderContext");
+      p = g.data_ptr<float>();
+    }
+    check_rc(gs_ctx_set_camera_grad(ctx, p), "gs_ctx_set_camera_grad");
+  }
+
   void set_timing(bool on) { check_rc(gs_ctx_set_timing(ctx, on ? 1 : 0), "gs_ctx_set_timing"); }
   std::vector<float> stage_ms() {
     std::vector<float> v(GS_N_STAGES, -1.f);
@@ -686,6 +700,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
       .def("set_timing", &RenderContext::set_timing)
       .def("set_grad_push", &RenderContext::set_grad_push)
       .def("clear_grad_push", &RenderContext::clear_grad_push)
+      .def("set_camera_grad", &RenderContext::set_camera_grad, py::arg("grad_cam"))
       .def("stage_ms", &RenderContext::stage_ms)
       .def("sorted_instances", &RenderContext::sorted_instances)
       .def("tile_consumed", &RenderContext::tile_consumed);

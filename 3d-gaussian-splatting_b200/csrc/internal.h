@@ -116,7 +116,12 @@ cudaError_t gs_launch_fused_project_bwd(const float* pos, const float* rgb, cons
                                         const uint32_t* count, const float* grad_inst, const uint32_t* row_epoch, uint32_t epoch,
                                         float* g_pos, float* g_rgb, float* g_opa,
                                         float* g_quat, float* g_scale, const GsGradPush& push, cudaStream_t st,
-                                        bool depth_grad = false /*maps frame: chain float 9 of the rows to pos*/);
+                                        bool depth_grad = false /*maps frame: chain float 9 of the rows to pos*/,
+                                        double* cam_partial = nullptr /*camera gradient: [blocks][12] partial rows*/);
+// Camera gradient (gs_ctx_set_camera_grad; RGB, one GPU): bytes of the partial rows the projection backward of n
+// Gaussians writes, and the one-block kernel that sums them in a fixed order into grad_cam[12] (zeros when n == 0).
+size_t gs_camgrad_partial_bytes(int n);
+cudaError_t gs_launch_camgrad_finish(const double* cam_partial, int n, float* grad_cam, cudaStream_t st);
 
 // ---- binning.cu ------------------------------------------------------------------------
 cudaError_t gs_launch_emit_keys(const GsRec* rec, const uint32_t* perm, const uint32_t* offsets_sorted, int n, int ntx,

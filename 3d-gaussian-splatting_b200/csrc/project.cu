@@ -140,9 +140,31 @@ __device__ __forceinline__ void push_store(const GsGradPush& P, float* local, co
   }
 }
 
+// Sum of the 12 camera-gradient floats of the block's 256 Gaussians, in double, in a fixed order (xor butterfly in
+// each warp, then warps 0..7): one partial row per block, partial[blockIdx.x][12].
+__device__ __forceinline__ void camgrad_block_reduce(const float gcam[12], double* __restrict__ partial) {
+  __shared__ double red[kBlock / 32][12];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int k = 0; k < 12; ++k) {
+    double v = (double)gcam[k];
+#pragma unroll
+    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if (lane == 0) red[warp][k] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x < 12) {
+    double s = 0.0;
+#pragma unroll
+    for (int w = 0; w < kBlock / 32; ++w) s += red[w][threadIdx.x];
+    partial[(size_t)blockIdx.x * 12 + threadIdx.x] = s;
+  }
+}
+
 // DEPTH (maps frames, D == 3): float 9 of the rows is d/d|p_c| and is chained to pos; otherwise the depth is only a
-// sort key.
-template <int D, int GW, int W, bool DEPTH = false>
+// sort key.  CAMGRAD (RGB, one GPU): also the camera gradient of the block's Gaussians, one partial row per block
+// into cam_partial (summed by camgrad_finish_kernel); every thread of the block takes part in that reduction.
+template <int D, int GW, int W, bool DEPTH = false, bool CAMGRAD = false>
 __global__ void __launch_bounds__(kBlock) fused_project_bwd_kernel(
     const float* __restrict__ pos, const float* __restrict__ rgb, const float* __restrict__ opa,
     const float* __restrict__ quat, const float* __restrict__ scale, int n, int scale_act, GsCam cam,
@@ -150,13 +172,17 @@ __global__ void __launch_bounds__(kBlock) fused_project_bwd_kernel(
     const uint32_t* __restrict__ count, const float* __restrict__ grad_inst,
     const uint32_t* __restrict__ row_epoch, uint32_t epoch, float* __restrict__ g_pos,
     float* __restrict__ g_rgb, float* __restrict__ g_opa, float* __restrict__ g_quat, float* __restrict__ g_scale,
-    GsGradPush push) {
+    GsGradPush push, double* __restrict__ cam_partial) {
+  static_assert(!CAMGRAD || (D == 3 && W == 0), "camera gradients: RGB colour on one GPU only");
   int i = blockIdx.x * kBlock + threadIdx.x;
   // SH colour on one GPU: the warp writes its coefficient gradients together (below), so threads past n stay
   constexpr bool kStagedRgb = (D != 3) && (W == 0);
   const bool valid = i < n;
-  if (!valid && !kStagedRgb) return;
+  if (!valid && !kStagedRgb && !CAMGRAD) return;
   float gp[3] = {0.f, 0.f, 0.f}, gq_raw[4] = {0.f, 0.f, 0.f, 0.f}, gs_raw[3] = {0.f, 0.f, 0.f};
+  float gcam[12];
+#pragma unroll
+  for (int k = 0; k < 12; ++k) gcam[k] = 0.f;
   float go = 0.f;
   float acc[GW];
 #pragma unroll
@@ -204,7 +230,7 @@ __global__ void __launch_bounds__(kBlock) fused_project_bwd_kernel(
     static_assert(!DEPTH || D == 3, "the depth gradient has a row slot in the RGB layout only");
     float gxyd[3] = {acc[0], acc[1], DEPTH ? acc[9] : 0.f};   // depth: sort key, + map gradient in maps frames
     float gq[4], gsv[3];
-    gs_project_backward(cam, p, q, s, gxyd, gcov, gp, gq, gsv);
+    gs_project_backward(cam, p, q, s, gxyd, gcov, gp, gq, gsv, CAMGRAD ? gcam : nullptr);
     // quat normalisation backward: q = r/|r|
     float dot = q[0] * gq[0] + q[1] * gq[1] + q[2] * gq[2] + q[3] * gq[3];
 #pragma unroll
@@ -227,7 +253,9 @@ __global__ void __launch_bounds__(kBlock) fused_project_bwd_kernel(
       }
     }
   }
-  if (W == 0) {
+  if (CAMGRAD && !valid) {
+    // past n: no rows to store, zeros to the camera-gradient reduction below
+  } else if (W == 0) {
     if constexpr (kStagedRgb) {
       // The 32 Gaussians of a warp own 32 * D contiguous floats of g_rgb.  One strided 4-byte store per coefficient
       // makes every store a partial-sector write (read-modify-write under ECC: 8x the bytes; 0.45 / 0.91 ms at
@@ -276,6 +304,20 @@ __global__ void __launch_bounds__(kBlock) fused_project_bwd_kernel(
         make_float4(gq_raw[0], gq_raw[1], gq_raw[2], gq_raw[3]);
     push_store<W, 1>(push, g_opa + i, &go);
   }
+  if constexpr (CAMGRAD) camgrad_block_reduce(gcam, cam_partial);
+}
+
+// Sums the partial rows of the projection backward in block order, in double: warp k owns float k of the camera
+// gradient (lane stride over the rows, then a fixed xor butterfly).  No atomics: bit-deterministic.  nblocks == 0
+// (no Gaussian) writes zeros.
+__global__ void __launch_bounds__(12 * 32) camgrad_finish_kernel(const double* __restrict__ partial, int nblocks,
+                                                                 float* __restrict__ out) {
+  const int k = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  double s = 0.0;
+  for (int b = lane; b < nblocks; b += 32) s += partial[(size_t)b * 12 + k];
+#pragma unroll
+  for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  if (lane == 0) out[k] = (float)s;
 }
 
 }  // namespace
@@ -439,20 +481,29 @@ cudaError_t gs_launch_fused_project_bwd(const float* pos, const float* rgb, cons
                                         const uint32_t* count, const float* grad_inst, const uint32_t* row_epoch, uint32_t epoch,
                                         float* g_pos, float* g_rgb, float* g_opa,
                                         float* g_quat, float* g_scale, const GsGradPush& push, cudaStream_t st,
-                                        bool depth_grad) {
+                                        bool depth_grad, double* cam_partial) {
   if (n == 0) return cudaSuccess;
-  if (depth_grad) {
-    if (d != 3 || push.world != 0) return cudaErrorInvalidValue;
-    fused_project_bwd_kernel<3, GS_GREC, 0, true><<<grid_for(n), kBlock, 0, st>>>(
-        pos, rgb, opa, quat, scale, n, scale_act, cam, near_plane, half_w, half_h, offsets_g, count, grad_inst, row_epoch,
-        epoch, g_pos, g_rgb, g_opa, g_quat, g_scale, push);
+  if (cam_partial && (d != 3 || push.world != 0)) return cudaErrorInvalidValue;
+#define GS_LAUNCH_PBWD_RGB(DEPTH, CAMGRAD)                                                                          \
+  fused_project_bwd_kernel<3, GS_GREC, 0, DEPTH, CAMGRAD><<<grid_for(n), kBlock, 0, st>>>(                         \
+      pos, rgb, opa, quat, scale, n, scale_act, cam, near_plane, half_w, half_h, offsets_g, count, grad_inst,       \
+      row_epoch, epoch, g_pos, g_rgb, g_opa, g_quat, g_scale, push, cam_partial)
+  if (cam_partial) {
+    if (depth_grad) GS_LAUNCH_PBWD_RGB(true, true);
+    else GS_LAUNCH_PBWD_RGB(false, true);
     return cudaGetLastError();
   }
+  if (depth_grad) {
+    if (d != 3 || push.world != 0) return cudaErrorInvalidValue;
+    GS_LAUNCH_PBWD_RGB(true, false);
+    return cudaGetLastError();
+  }
+#undef GS_LAUNCH_PBWD_RGB
 #define GS_LAUNCH_PBWD(D, GW, W)                                                                                    \
   fused_project_bwd_kernel<D, GW, W><<<grid_for(n), kBlock, 0, st>>>(pos, rgb, opa, quat, scale, n, scale_act, cam, \
                                                                      near_plane, half_w, half_h, offsets_g, count, \
                                                                      grad_inst, row_epoch, epoch, g_pos, g_rgb,    \
-                                                                     g_opa, g_quat, g_scale, push)
+                                                                     g_opa, g_quat, g_scale, push, nullptr)
 #define GS_LAUNCH_PBWD_W(D, GW)                  \
   switch (push.world) {                          \
     case 0: GS_LAUNCH_PBWD(D, GW, 0); break;     \
@@ -466,5 +517,12 @@ cudaError_t gs_launch_fused_project_bwd(const float* pos, const float* rgb, cons
   else { GS_LAUNCH_PBWD_W(48, 56) }
 #undef GS_LAUNCH_PBWD_W
 #undef GS_LAUNCH_PBWD
+  return cudaGetLastError();
+}
+
+size_t gs_camgrad_partial_bytes(int n) { return (size_t)grid_for(n) * 12 * sizeof(double); }
+
+cudaError_t gs_launch_camgrad_finish(const double* cam_partial, int n, float* grad_cam, cudaStream_t st) {
+  camgrad_finish_kernel<<<1, 12 * 32, 0, st>>>(cam_partial, n > 0 ? grid_for(n) : 0, grad_cam);
   return cudaGetLastError();
 }

@@ -83,11 +83,13 @@ __device__ __forceinline__ GsProj gs_project(const GsCam& cam, const float p[3],
 
 // Backward of gs_project for a visible Gaussian.  g_xyd = dL/d(x/z, y/z, depth),
 // g_cov = dL/d(a,b,c,d).  Outputs dL/dp (world), dL/dq (wrt the NORMALISED quaternion
-// entries as independent variables, like the reference), dL/ds (activated scale).
+// entries as independent variables, like the reference), dL/ds (activated scale) and, when
+// gcam is non-null, this Gaussian's share of dL/d(cam.r[9], cam.t[3]) (12 floats, written):
+// p_c = R p + t and JW = J R with J detached, as for every other gradient here.
 __device__ __forceinline__ void gs_project_backward(const GsCam& cam, const float p[3], const float q[4],
                                                     const float s[3], const float g_xyd[3],
                                                     const float g_cov[4], float gp[3], float gq[4],
-                                                    float gs[3]) {
+                                                    float gs[3], float* gcam = nullptr) {
   float pc[3];
   gs_world_to_cam(cam, p, pc);
   float r = sqrtf(pc[0] * pc[0] + pc[1] * pc[1] + pc[2] * pc[2]);
@@ -122,6 +124,31 @@ __device__ __forceinline__ void gs_project_backward(const GsCam& cam, const floa
   for (int rr = 0; rr < 3; ++rr)
 #pragma unroll
     for (int c = 0; c < 3; ++c) grs[rr * 3 + c] = jw0[rr] * h0[c] + jw1[rr] * h1[c];
+  if (gcam) {
+    // mean: dL/dt = gc, dL/dR[a][b] = gc[a] p[b].  Covariance: dL/d(JW)[r][k] = sum_c h_r[c] RS[k][c], chained
+    // through the image-plane rows (iz, 0, jx), (0, iz, jy) of J (gs_jw_rows).
+    const float jx = -pc[0] / (pc[2] * pc[2]);
+    const float jy = -pc[1] / (pc[2] * pc[2]);
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      gcam[9 + a] = gc[a];
+#pragma unroll
+      for (int b = 0; b < 3; ++b) gcam[a * 3 + b] = gc[a] * p[b];
+    }
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      float gjw0 = 0.f, gjw1 = 0.f;
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        const float rs = R.m[k * 3 + c] * s[c];
+        gjw0 += h0[c] * rs;
+        gjw1 += h1[c] * rs;
+      }
+      gcam[k] += iz * gjw0;
+      gcam[3 + k] += iz * gjw1;
+      gcam[6 + k] += jx * gjw0 + jy * gjw1;
+    }
+  }
   float gR[9];
 #pragma unroll
   for (int c = 0; c < 3; ++c) {

@@ -146,6 +146,7 @@ struct gs_ctx {
   uint32_t epoch = 0;                      // tag of the current backward in row_epoch[]
   // per tile / misc
   DevBuf tile_accum, tile_neff, tile_neff_b, cub_tmp, counters, img_dev, gimg_dev, rays;
+  DevBuf cam_partial;                     // camera gradient: one [12] double row per projection-backward block
   float* host_rays = nullptr;             // pinned: rays_o, lefttop, dx, dy (SH colour only)
   unsigned long long* host_m = nullptr;   // pinned: {M}
   cudaEvent_t ev_m = nullptr;             // marks the completion of the M read-back
@@ -166,6 +167,8 @@ struct gs_ctx {
   bool ev_fwd_valid = false, ev_bwd_valid = false;
   // data-parallel gradient push (gs_ctx_set_grad_push); world == 0: off
   GsGradPush push{};
+  // camera gradient output (gs_ctx_set_camera_grad; device, 12 floats); nullptr: off
+  float* grad_cam = nullptr;
 };
 
 // stage boundaries: event i is recorded BEFORE stage i; stage i lasts ev[i+1]-ev[i]
@@ -199,7 +202,7 @@ extern "C" void gs_ctx_destroy(gs_ctx* c) {
   cudaDeviceSynchronize();
   DevBuf* bufs[] = {&c->rec, &c->count, &c->offsets, &c->dkey_in, &c->dkey_out, &c->perm, &c->iota, &c->offsets_g, &c->keys_in, &c->keys_out,
                     &c->vals_in, &c->vals_out, &c->pA, &c->pB, &c->pC, &c->grad_inst, &c->row_epoch, &c->tile_accum, &c->tile_neff,
-                    &c->tile_neff_b, &c->cub_tmp, &c->counters, &c->img_dev, &c->gimg_dev, &c->rays};
+                    &c->tile_neff_b, &c->cub_tmp, &c->counters, &c->img_dev, &c->gimg_dev, &c->rays, &c->cam_partial};
   for (DevBuf* b : bufs) b->release();
   if (c->host_m) cudaFreeHost(c->host_m);
   if (c->host_rays) cudaFreeHost(c->host_rays);
@@ -239,6 +242,20 @@ static int check_maps_supported(const gs_ctx* c, int d, const char* fn) {
     why = "depth / alpha maps need the gather path (gs_tune(\"gather\", 0) is set)";
   else if (c->push.world != 0)
     why = "depth / alpha maps do not support the data-parallel gradient push (gs_ctx_set_grad_push is active)";
+  if (!why) return 0;
+  snprintf(msg, sizeof(msg), "%s: %s", fn, why);
+  return gs_set_error_msg(GS_ERR_UNSUPPORTED, msg);
+}
+
+// camera gradients need RGB colour on one GPU; returns 0 or the refusal
+static int check_camgrad_supported(const gs_ctx* c, const char* fn) {
+  char msg[260];
+  const char* why = nullptr;
+  if (c->d != 3)
+    why = "camera gradients need RGB colour (d == 3); with SH colour the per-pixel SH basis depends on the camera "
+          "through the ray directions, which is not differentiated";
+  else if (c->push.world != 0)
+    why = "camera gradients do not support the data-parallel gradient push (gs_ctx_set_grad_push is active)";
   if (!why) return 0;
   snprintf(msg, sizeof(msg), "%s: %s", fn, why);
   return gs_set_error_msg(GS_ERR_UNSUPPORTED, msg);
@@ -511,6 +528,8 @@ static int render_backward_impl(gs_ctx* c, const float* pos, const float* rgb, c
                                 float* grad_scale, gs_stream_t stream, const GsMapsBwd* maps = nullptr) {
   if (!c) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_render_backward: null ctx");
   if (!c->have_forward) return gs_set_error_msg(GS_ERR_NO_FORWARD, "gs_render_backward: no forward on this ctx");
+  if (c->grad_cam)
+    if (int rc = check_camgrad_supported(c, maps ? "gs_render_backward_maps" : "gs_render_backward")) return rc;
   if (maps) {
     if (!c->maps)
       return gs_set_error_msg(GS_ERR_NO_FORWARD,
@@ -529,6 +548,7 @@ static int render_backward_impl(gs_ctx* c, const float* pos, const float* rgb, c
   const int d = c->d;
   const size_t grow = d == 3 ? (size_t)GS_GREC * 4 : (size_t)gs_sh_grad_width(d) * 4;
   GS_CUDA_TRY(c->grad_inst.reserve(M * grow + 16, st));
+  if (c->grad_cam) GS_CUDA_TRY(c->cam_partial.reserve(gs_camgrad_partial_bytes(c->n), st));
   {
     // one u32 tag per gradient row: rows written by this backward carry `epoch`; the tails of
     // saturated tiles are never written nor read (saves ~0.2 GB of HBM writes + reads at C3)
@@ -587,8 +607,12 @@ static int render_backward_impl(gs_ctx* c, const float* pos, const float* rgb, c
                                           c->half_w, c->half_h, c->offsets_g.as<uint32_t>(), c->count.as<uint32_t>(),
                                           c->grad_inst.as<float>(), c->row_epoch.as<uint32_t>(), c->epoch,
                                           grad_pos, grad_rgb, grad_opa, grad_quat, grad_scale, c->push, st,
-                                          maps != nullptr));
+                                          maps != nullptr, c->grad_cam ? c->cam_partial.as<double>() : nullptr));
   if (c->n > 0) gs_count_launch();
+  if (c->grad_cam) {
+    GS_CUDA_TRY(gs_launch_camgrad_finish(c->cam_partial.as<double>(), c->n, c->grad_cam, st));
+    gs_count_launch();
+  }
   gs_mark(c, 9, st);
   c->ev_bwd_valid = c->timing && c->ev_ok;
   return 0;
@@ -664,6 +688,15 @@ extern "C" int gs_ctx_set_grad_push(gs_ctx* c, const gs_grad_push* p) {
     g.staging[k] = p->staging[k];
   }
   c->push = g;
+  return 0;
+}
+
+extern "C" int gs_ctx_set_camera_grad(gs_ctx* c, float* grad_cam) {
+  // the pointer is checked first so that both refusals need no context
+  if (reinterpret_cast<uintptr_t>(grad_cam) % alignof(float))
+    return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_ctx_set_camera_grad: grad_cam must be 4-byte aligned");
+  if (!c) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_ctx_set_camera_grad: null ctx");
+  c->grad_cam = grad_cam;
   return 0;
 }
 

@@ -6,7 +6,8 @@ conventions as reference renderer.py (`draw` :89, `trunc_exp` :102,
 reference keeps working; underneath, every op calls the sm_100a kernels of
 libgs_b200 through the `gaussian` extension in this directory.  Additive:
 `render_frame`, one autograd node for the whole frame (fused path), and `render_frame_maps`,
-the same frame with depth / alpha maps and a background colour.
+the same frame with depth / alpha maps and a background colour.  All three frames also differentiate
+the camera pose (`rot`, `tran`) when a pose tensor requires grad (RGB colour only).
 
 The product path never falls back to PyTorch/CPU math: importing this module
 without the built extension raises.
@@ -187,6 +188,34 @@ def _apply_push(rctx, push):
         rctx.set_grad_push(*push)
 
 
+# positions of rot / tran among the inputs of the three frame Functions (ctx.needs_input_grad)
+_ROT, _TRAN = 10, 11
+
+
+def _save_pose(ctx, rot, tran):
+    ctx.pose = [(t.shape, t.dtype, t.device) if isinstance(t, torch.Tensor) else None for t in (rot, tran)]
+
+
+def _backward_with_pose(ctx, pos, run):
+    """Runs `run()` (the context's backward); when rot or tran needs a gradient, the same backward also writes the
+    camera gradient (gs_ctx_set_camera_grad, one more kernel), returned as (grad_rot, grad_tran) in each input's
+    shape, dtype and device.  Otherwise nothing changes and (None, None) is returned."""
+    want = [ctx.needs_input_grad[_ROT], ctx.needs_input_grad[_TRAN]]
+    if not any(want):
+        run()
+        return None, None
+    gcam = torch.empty(12, device=pos.device, dtype=torch.float32)
+    ctx.rctx.set_camera_grad(gcam)
+    try:
+        run()
+    finally:
+        ctx.rctx.set_camera_grad(None)
+    out = []
+    for w, part, meta in zip(want, (gcam[:9], gcam[9:]), ctx.pose):
+        out.append(part.reshape(meta[0]).to(dtype=meta[1], device=meta[2]) if w else None)
+    return tuple(out)
+
+
 class _RenderFrame(torch.autograd.Function):
     """raw parameters -> padded un-clamped image, replacing splatter.py:513-634's glue.
 
@@ -203,6 +232,7 @@ class _RenderFrame(torch.autograd.Function):
                                    float(tile_thresh), SCALE_ACTIVATIONS[scale_activation])
         ctx.rctx = rctx
         ctx.frame = rctx.frame_id()
+        _save_pose(ctx, rot, tran)
         ctx.save_for_backward(pos, rgb, opa, quat, scale, image)
         ctx.mark_non_differentiable(mask)
         return image, mask
@@ -212,8 +242,10 @@ class _RenderFrame(torch.autograd.Function):
         pos, rgb, opa, quat, scale, image = ctx.saved_tensors
         outs, push = _flat_grads((pos, rgb, opa, quat, scale))
         _apply_push(ctx.rctx, push)
-        ctx.rctx.backward_into(pos, rgb, opa, quat, scale, image, _f32(grad_image), *outs, ctx.frame)
-        return (None, outs[0], outs[1], outs[2], outs[3], outs[4]) + (None,) * 9
+        g_rot, g_tran = _backward_with_pose(
+            ctx, pos, lambda: ctx.rctx.backward_into(pos, rgb, opa, quat, scale, image, _f32(grad_image), *outs,
+                                                     ctx.frame))
+        return (None, outs[0], outs[1], outs[2], outs[3], outs[4]) + (None,) * 4 + (g_rot, g_tran) + (None,) * 3
 
 
 render_frame = _RenderFrame.apply
@@ -233,6 +265,7 @@ class _RenderFrameFinal(torch.autograd.Function):
                                               float(tile_thresh), SCALE_ACTIVATIONS[scale_activation])
         ctx.rctx = rctx
         ctx.frame = rctx.frame_id()
+        _save_pose(ctx, rot, tran)
         ctx.save_for_backward(pos, rgb, opa, quat, scale, raw)
         ctx.mark_non_differentiable(mask)
         return final, mask
@@ -242,8 +275,10 @@ class _RenderFrameFinal(torch.autograd.Function):
         pos, rgb, opa, quat, scale, raw = ctx.saved_tensors
         outs, push = _flat_grads((pos, rgb, opa, quat, scale))
         _apply_push(ctx.rctx, push)
-        ctx.rctx.backward_final_into(pos, rgb, opa, quat, scale, raw, _f32(grad_final), *outs, ctx.frame)
-        return (None, outs[0], outs[1], outs[2], outs[3], outs[4]) + (None,) * 9
+        g_rot, g_tran = _backward_with_pose(
+            ctx, pos, lambda: ctx.rctx.backward_final_into(pos, rgb, opa, quat, scale, raw, _f32(grad_final), *outs,
+                                                           ctx.frame))
+        return (None, outs[0], outs[1], outs[2], outs[3], outs[4]) + (None,) * 4 + (g_rot, g_tran) + (None,) * 3
 
 
 render_frame_final = _RenderFrameFinal.apply
@@ -265,6 +300,7 @@ class _RenderFrameMaps(torch.autograd.Function):
             bool(final))
         ctx.rctx = rctx
         ctx.frame = rctx.frame_id()
+        _save_pose(ctx, rot, tran)
         ctx.final = bool(final)
         ctx.save_for_backward(pos, rgb, opa, quat, scale, raw, draw_, araw)
         ctx.mark_non_differentiable(mask)
@@ -276,9 +312,11 @@ class _RenderFrameMaps(torch.autograd.Function):
         pos, rgb, opa, quat, scale, raw, draw_, araw = ctx.saved_tensors
         outs, push = _flat_grads((pos, rgb, opa, quat, scale))
         _apply_push(ctx.rctx, push)
-        ctx.rctx.backward_maps_into(pos, rgb, opa, quat, scale, raw, draw_, araw, _f32(grad_image), _f32(grad_depth),
-                                    _f32(grad_alpha), ctx.final, *outs, ctx.frame)
-        return (None, outs[0], outs[1], outs[2], outs[3], outs[4]) + (None,) * 11
+        g_rot, g_tran = _backward_with_pose(
+            ctx, pos, lambda: ctx.rctx.backward_maps_into(pos, rgb, opa, quat, scale, raw, draw_, araw,
+                                                          _f32(grad_image), _f32(grad_depth), _f32(grad_alpha),
+                                                          ctx.final, *outs, ctx.frame))
+        return (None, outs[0], outs[1], outs[2], outs[3], outs[4]) + (None,) * 4 + (g_rot, g_tran) + (None,) * 5
 
 
 def render_frame_maps(rctx, pos, rgb, opa, quat, scale, width, height, focal_x, focal_y, rot, tran, near,

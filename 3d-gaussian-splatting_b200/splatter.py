@@ -245,12 +245,18 @@ class Splatter(nn.Module):
 
     # -- camera -----------------------------------------------------------------------------
     def set_camera(self, idx, extrinsics=None, intrinsics=None):
-        """reference splatter.py:465-511 (idx=None: free camera from the GUI)."""
+        """reference splatter.py:465-511 (idx=None: free camera from the GUI).  On the free-camera path, torch
+        tensors in `extrinsics` reach the renderer as they are, so a pose that requires grad receives gradients
+        (pose refinement; the kernels get a host copy); other array types become constant float32 host tensors.
+        Views addressed by index keep their stored constant pose."""
         if idx is None:
+            def pose(x):
+                if isinstance(x, torch.Tensor):
+                    return x
+                return torch.as_tensor(np.asarray(x), dtype=torch.float32).cpu().contiguous()
             v = dict(width=int(math.ceil(intrinsics["width"])), height=int(math.ceil(intrinsics["height"])),
                      focal_x=float(intrinsics["focal_x"]), focal_y=float(intrinsics["focal_y"]),
-                     rot=torch.as_tensor(np.asarray(extrinsics["rot"]), dtype=torch.float32).cpu().contiguous(),
-                     tran=torch.as_tensor(np.asarray(extrinsics["tran"]), dtype=torch.float32).cpu().contiguous())
+                     rot=pose(extrinsics["rot"]), tran=pose(extrinsics["tran"]))
             self.ground_truth = None
         else:
             v = self.views[idx]

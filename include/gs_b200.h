@@ -221,6 +221,23 @@ int gs_render_backward_maps(gs_ctx* ctx, const float* pos, const float* rgb, con
                             int grad_is_final, float* grad_pos, float* grad_rgb, float* grad_opa,
                             float* grad_quat, float* grad_scale, gs_stream_t stream);
 
+/* New (an extension; the reference treats the camera as a constant): camera pose gradients.  While grad_cam is set
+ * (a DEVICE pointer to 12 floats, 4-byte aligned; NULL clears it), every gs_render_backward, gs_render_backward_final
+ * and gs_render_backward_maps on ctx also overwrites grad_cam with the gradient of the same L as the parameter
+ * gradients (<grad_image, image>, plus <grad_depth, depth> + <grad_alpha, alpha> for a maps frame) wrt the camera of
+ * ctx's last forward:
+ *   grad_cam[0..9)  = dL/d rot   (row-major; the 9 entries as independent variables, no SO(3) projection: chain it to
+ *                                 a quaternion / axis-angle parametrisation on the caller's side)
+ *   grad_cam[9..12) = dL/d tran
+ * Conventions as for the parameters: the projection Jacobian J is detached (p_c = R p + t and J R both carry R), the
+ * 1.2x frustum cull, the near plane, the tile binning and the sort order are constants, and in plain frames the depth
+ * is a sort key only (maps frames add the depth map's d_i = |R p_i + t|).  Deterministic (no atomics); the backward
+ * launches one more kernel.  A frame without instances writes zeros.  Refused at backward time with
+ * GS_ERR_UNSUPPORTED (reason in gs_last_error) for d != 3 (SH colour: the per-pixel SH basis depends on the camera
+ * through the ray directions, which is not differentiated) and while a gs_ctx_set_grad_push configuration is active,
+ * whichever of the two was set first.  GS_ERR_INVALID_ARG for a null ctx or a misaligned pointer. */
+int gs_ctx_set_camera_grad(gs_ctx* ctx, float* grad_cam);
+
 /* Per-stage device timing with CUDA events recorded on the frame's stream (off by default).
  * gs_frame_stage_ms fills out[GS_N_STAGES] with the milliseconds of the last frame's stages:
  * 0 project, 1 depth sort of Gaussians + scan + M readback, 2 key emit, 3 tile-id radix sort,
