@@ -716,13 +716,13 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("loss_l1_ssim", &loss_l1_ssim, "fused L1 + SSIM loss, forward + image gradient (CUDA)");
   m.def("adam_step", &adam_step, "fused Adam over flat parameter / gradient buffers (CUDA)");
   m.def("tune", [](const std::string& name, int value) { check_rc(gs_tune(name.c_str(), value), "gs_tune"); },
-        "set an A/B tuning knob of the blend kernels (see include/gs_b200.h gs_tune)");
+        "set a blend-path knob: gather (0 packed, 1 gather) or sh_tc (0..3); see include/gs_b200.h gs_tune");
   m.def("tuned", [](const std::string& name) {
           int v = 0;
           check_rc(gs_tune_get(name.c_str(), &v), "gs_tune_get");
           return v;
         },
-        "current value of an A/B tuning knob of the blend kernels");
+        "current value of a gs_tune knob (gather, sh_tc)");
   m.def("kernel_launches", []() { return (int64_t)gs_kernel_launches(); },
         "kernels of libgs_b200 launched by this process so far");
   m.attr("abi_version") = gs_abi_version();

@@ -12,9 +12,9 @@
 //     no FP64, no division in the forward loop;
 //   * whole-warp and whole-CTA early exit once every pixel is saturated, so a tile's tail is
 //     never read (M_eff accounting);
-//   * backward: 64 threads x 4 pixels per tile; 9 moment sums per instance are reduced with a
-//     recursive-halving shuffle network (14 SHFL instead of 45), combined across the two warps
-//     through shared memory and written as ONE record per instance (no atomics, deterministic).
+//   * backward: one warp x 8 pixels per thread per tile; six partial sums per (thread, instance) go to shared
+//     memory and a second phase of 4 threads per instance reduces them and writes ONE record per instance
+//     (no atomics, deterministic).
 #include <cstdlib>
 #include <type_traits>
 
@@ -25,19 +25,12 @@ namespace {
 // =======================================================================================
 // forward
 // =======================================================================================
-constexpr int FWD_THREADS = 64;    // 2 warps per tile; each thread owns a row of 4 adjacent pixels
-constexpr int FWD_PX = 4;
+constexpr int FWD_CH = 128;                  // instances per staging chunk
+constexpr int FWD_PX = 4;                    // each thread owns a row of 4 adjacent pixels
+constexpr int FWD_THREADS = 256 / FWD_PX;    // 2 warps per tile
 constexpr int FWD_STAGES = 2;
 
-template <int FWD_CH>
-struct FwdSmem {
-  float4 A[FWD_STAGES][FWD_CH];
-  float4 C[FWD_STAGES][FWD_CH];
-  float2 B[FWD_STAGES][FWD_CH + 2];
-  uint64_t full[FWD_STAGES];
-};
-
-template <typename SM, int CH>
+template <typename SM>
 __device__ __forceinline__ void issue_chunk(SM& sm, int stage, const float4* __restrict__ pA,
                                             const float2* __restrict__ pB, const float4* __restrict__ pC,
                                             int base, int n, int shift) {
@@ -57,6 +50,14 @@ __device__ __forceinline__ void issue_chunk(SM& sm, int stage, const float4* __r
 //          cp.async pieces of the Gaussian's record straight from GsRec rec[N] through the sorted id list and
 //          arrives on the stage's mbarrier when they have landed (cp.async.mbarrier.arrive; barrier count = CTA
 //          threads).  The per-instance record in shared memory is {a, b, c, d} (gs_common.cuh GsRec).
+template <int CH, int STAGES>
+struct PackedRing {
+  float4 A[STAGES][CH];
+  float4 C[STAGES][CH];
+  float2 B[STAGES][CH + 2];
+  uint64_t full[STAGES];
+};
+
 template <bool GATHER>
 struct StageView;
 template <>
@@ -142,10 +143,9 @@ __device__ __forceinline__ void gather_issue(SM& sm, int stage, const GsRec* __r
 // + 4 pixels x (dx, u, exponent, MUFU.EX2, setp, mul, sel, 3 FFMA colour, T update) = 12.75
 // issue slots per (pixel, instance) instead of 17-18 with one pixel per thread.
 // MAPS (gather path only): one more FFMA per (pixel, instance) accumulates the depth map; the epilogue adds T * bg to
-// the colour and stores depth and alpha = 1 - T.  `maps` is the last parameter so that the other instantiations keep
-// their parameter offsets (and their code).
-template <int FWD_CH, int PX, bool GATHER, bool MAPS = false>
-__global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __restrict__ pA,
+// the colour and stores depth and alpha = 1 - T.
+template <bool GATHER, bool MAPS>
+__global__ void __launch_bounds__(FWD_THREADS) blend_fwd_kernel(const float4* __restrict__ pA,
                                                                  const float2* __restrict__ pB,
                                                                  const float4* __restrict__ pC,
                                                                  const GsRec* __restrict__ grec,
@@ -155,15 +155,16 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
                                                                  float* __restrict__ image,
                                                                  int* __restrict__ tile_neff,
                                                                  float* __restrict__ final_img, GsCrop crop,
-                                                                 GsMapsFwd maps = GsMapsFwd{}) {
+                                                                 GsMapsFwd maps) {
   static_assert(!MAPS || GATHER, "depth / alpha maps read the depth from the gathered records");
-  using Smem = typename std::conditional<GATHER, GatherRing<FWD_CH, FWD_STAGES, 3>, FwdSmem<FWD_CH>>::type;
+  using Smem =
+      typename std::conditional<GATHER, GatherRing<FWD_CH, FWD_STAGES, 3>, PackedRing<FWD_CH, FWD_STAGES>>::type;
   __shared__ __align__(16) Smem sm;
   const int tile = blockIdx.x;
   const int tid = threadIdx.x;
   const int tx = tile % ntx, ty = tile / ntx;
-  // thread -> a row of PX adjacent pixels (ix0 .. ix0+PX-1, iy); PX = 4: 2 warps per tile, 8: one warp
-  constexpr int FWD_PX = PX, TPR = GS_TILE / PX, NTHREADS = 256 / PX;
+  // thread -> a row of FWD_PX adjacent pixels (ix0 .. ix0+FWD_PX-1, iy)
+  constexpr int TPR = GS_TILE / FWD_PX;
   const int ix0 = tx * GS_TILE + (tid % TPR) * FWD_PX;
   const int iy = ty * GS_TILE + (tid / TPR);
   float px[FWD_PX];
@@ -177,20 +178,20 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
   const int nchunks = (cnt + FWD_CH - 1) / FWD_CH;
 
   if (tid == 0) {
-    for (int s = 0; s < FWD_STAGES; ++s) gs_mbar_init(&sm.full[s], GATHER ? NTHREADS : 1);
+    for (int s = 0; s < FWD_STAGES; ++s) gs_mbar_init(&sm.full[s], GATHER ? FWD_THREADS : 1);
     gs_fence_barrier_init();
   }
   __syncthreads();
-  GatherIds<NTHREADS, FWD_CH> gid;
+  GatherIds<FWD_THREADS, FWD_CH> gid;
   if constexpr (GATHER) {
     for (int k = 0; k < FWD_STAGES && k < nchunks; ++k) {
       gid.load(ids, start + k * FWD_CH, min(FWD_CH, cnt - k * FWD_CH), tid);
-      gather_issue<Smem, NTHREADS, FWD_CH, 3>(sm, k, grec, nullptr, gid, min(FWD_CH, cnt - k * FWD_CH), tid);
+      gather_issue<Smem, FWD_THREADS, FWD_CH, 3>(sm, k, grec, nullptr, gid, min(FWD_CH, cnt - k * FWD_CH), tid);
     }
     if (FWD_STAGES < nchunks) gid.load(ids, start + FWD_STAGES * FWD_CH, min(FWD_CH, cnt - FWD_STAGES * FWD_CH), tid);
   } else if (tid == 0) {
     for (int k = 0; k < FWD_STAGES && k < nchunks; ++k)
-      issue_chunk<Smem, FWD_CH>(sm, k, pA, pB, pC, start + k * FWD_CH, min(FWD_CH, cnt - k * FWD_CH), shift);
+      issue_chunk<Smem>(sm, k, pA, pB, pC, start + k * FWD_CH, min(FWD_CH, cnt - k * FWD_CH), shift);
   }
 
   float T[FWD_PX], cr[FWD_PX], cg[FWD_PX], cb[FWD_PX];
@@ -259,8 +260,7 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
     bool dead = true;
 #pragma unroll
     for (int p = 0; p < FWD_PX; ++p) dead = dead && !(T[p] > GS_T_STOP);
-    const int all_dead = NTHREADS == 32 ? __all_sync(0xffffffffu, dead) : __syncthreads_and(dead);
-    if (NTHREADS == 32) __syncwarp();
+    const int all_dead = __syncthreads_and(dead);
     if (all_dead) {
       consumed = min(cnt, (k + 1) * FWD_CH);
       break;
@@ -268,10 +268,10 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
     if (k + FWD_STAGES < nchunks) {
       const int kn = k + FWD_STAGES;            // every thread is past the barrier above: the stage is free
       if constexpr (GATHER) {
-        gather_issue<Smem, NTHREADS, FWD_CH, 3>(sm, stage, grec, nullptr, gid, min(FWD_CH, cnt - kn * FWD_CH), tid);
+        gather_issue<Smem, FWD_THREADS, FWD_CH, 3>(sm, stage, grec, nullptr, gid, min(FWD_CH, cnt - kn * FWD_CH), tid);
         if (kn + 1 < nchunks) gid.load(ids, start + (kn + 1) * FWD_CH, min(FWD_CH, cnt - (kn + 1) * FWD_CH), tid);
       } else if (tid == 0)
-        issue_chunk<Smem, FWD_CH>(sm, stage, pA, pB, pC, start + kn * FWD_CH, min(FWD_CH, cnt - kn * FWD_CH), shift);
+        issue_chunk<Smem>(sm, stage, pA, pB, pC, start + kn * FWD_CH, min(FWD_CH, cnt - kn * FWD_CH), shift);
     }
   }
   // drain copies that were issued but never consumed (early exit) before the CTA retires
@@ -280,7 +280,7 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
       gs_mbar_wait(&sm.full[kk % FWD_STAGES], (uint32_t)((kk / FWD_STAGES) & 1));
   }
   if constexpr (MAPS) {
-    // background behind the remaining transmittance; depth and alpha planes (PX floats = 16-byte aligned rows)
+    // background behind the remaining transmittance; depth and alpha planes (FWD_PX floats = 16-byte aligned rows)
     float av[FWD_PX];
 #pragma unroll
     for (int p = 0; p < FWD_PX; ++p) {
@@ -307,7 +307,7 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
       }
     }
   }
-  // PX pixels x 3 channels = PX * 12 contiguous, 16-byte aligned bytes
+  // FWD_PX pixels x 3 channels = FWD_PX * 12 contiguous, 16-byte aligned bytes
   {
     float ob[FWD_PX * 3];
 #pragma unroll
@@ -331,434 +331,48 @@ __global__ void __launch_bounds__(256 / PX) blend_fwd_kernel(const float4* __res
 // =======================================================================================
 // backward
 // =======================================================================================
-constexpr int BWD_STAGES = 2;
-constexpr int BWD_NV = 9;   // Sx Sy Sxx Sxy Syy S0 Cr Cg | Cb
-
-template <int WARPS, int BWD_CH>
-struct BwdSmem {
-  float4 A[BWD_STAGES][BWD_CH];
-  float4 C[BWD_STAGES][BWD_CH];
-  float2 B[BWD_STAGES][BWD_CH + 2];
-  uint64_t full[BWD_STAGES];
-  float partial[WARPS][BWD_CH * BWD_NV];
-};
-
-// WARPS warps per tile; every thread owns a row of PX = 8 / WARPS ... i.e. 256 / (32*WARPS)
-// horizontally adjacent pixels, so dy and every dy-only factor is shared by its pixels:
-// per pixel only S0 += e, Sx += e dx, Sxx += e dx^2 are accumulated and
-// Sy = dy S0, Sxy = dy Sx, Syy = dy^2 S0 are formed once per (thread, instance).
-template <int WARPS, int BWD_CH>
-__global__ void __launch_bounds__(32 * WARPS) blend_bwd_kernel(const float4* __restrict__ pA,
-                                                                const float2* __restrict__ pB,
-                                                                const float4* __restrict__ pC,
-                                                                const int* __restrict__ tile_accum, int wp, int hp,
-                                                                int ntx, float fx, float fy,
-                                                                const float* __restrict__ image,
-                                                                const float* __restrict__ grad_image,
-                                                                float* __restrict__ grad_inst, int grad_is_final,
-                                                                GsCrop crop, uint32_t* __restrict__ row_epoch,
-                                                                uint32_t epoch, int* __restrict__ tile_neff_b) {
-  constexpr int THREADS = 32 * WARPS;
-  constexpr int PX = 256 / THREADS;          // 8 (1 warp) or 4 (2 warps)
-  constexpr int TPR = GS_TILE / PX;          // threads per pixel row
-  using Smem = BwdSmem<WARPS, BWD_CH>;
-  __shared__ __align__(16) Smem sm;
-  const int tile = blockIdx.x;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int tx = tile % ntx, ty = tile / ntx;
-  const int start = tile_accum[tile];
-  const int cnt = tile_accum[tile + 1] - start;
-  if (cnt == 0) return;
-  const int shift = start & 1;
-  const int nchunks = (cnt + BWD_CH - 1) / BWD_CH;
-
-  const int ix0 = tx * GS_TILE + (tid % TPR) * PX;
-  const int iy = ty * GS_TILE + (tid / TPR);
-  float px[PX];
-#pragma unroll
-  for (int p = 0; p < PX; ++p) px[p] = gs_pixel_coord(ix0 + p, wp, fx);
-  const float py = gs_pixel_coord(iy, hp, fy);
-
-  float T[PX], R[PX], gr[PX], gg[PX], gb[PX];
-  {
-    const size_t off = ((size_t)iy * wp + ix0) * 3;     // PX*12 contiguous, 16-byte aligned bytes
-    const float4* im = reinterpret_cast<const float4*>(image + off);
-    float gbuf[PX * 3], ibuf[PX * 3];
-#pragma unroll
-    for (int q = 0; q < PX * 3 / 4; ++q) {
-      const float4 i4 = im[q];
-      ibuf[4 * q] = i4.x; ibuf[4 * q + 1] = i4.y; ibuf[4 * q + 2] = i4.z; ibuf[4 * q + 3] = i4.w;
-    }
-    if (!grad_is_final) {
-      const float4* gi = reinterpret_cast<const float4*>(grad_image + off);
-#pragma unroll
-      for (int q = 0; q < PX * 3 / 4; ++q) {
-        const float4 g4 = gi[q];
-        gbuf[4 * q] = g4.x; gbuf[4 * q + 1] = g4.y; gbuf[4 * q + 2] = g4.z; gbuf[4 * q + 3] = g4.w;
-      }
-    } else {
-#pragma unroll
-      for (int p = 0; p < PX; ++p)
-        gs_load_final_grad(grad_image, ibuf + 3 * p, ix0 + p, iy, crop.left, crop.top, crop.width, crop.height,
-                           gbuf[3 * p], gbuf[3 * p + 1], gbuf[3 * p + 2]);
-    }
-#pragma unroll
-    for (int p = 0; p < PX; ++p) {
-      gr[p] = gbuf[3 * p];
-      gg[p] = gbuf[3 * p + 1];
-      gb[p] = gbuf[3 * p + 2];
-      R[p] = gr[p] * ibuf[3 * p] + gg[p] * ibuf[3 * p + 1] + gb[p] * ibuf[3 * p + 2];
-      T[p] = 1.f;
-    }
-  }
-
-  if (tid == 0) {
-    for (int s = 0; s < BWD_STAGES; ++s) gs_mbar_init(&sm.full[s], 1);
-    gs_fence_barrier_init();
-  }
-  __syncthreads();
-  if (tid == 0) {
-    for (int k = 0; k < BWD_STAGES && k < nchunks; ++k)
-      issue_chunk<Smem, BWD_CH>(sm, k, pA, pB, pC, start + k * BWD_CH, min(BWD_CH, cnt - k * BWD_CH), shift);
-  }
-
-  int consumed = cnt;
-  int k = 0;
-  for (; k < nchunks; ++k) {
-    const int stage = k % BWD_STAGES;
-    gs_mbar_wait(&sm.full[stage], (uint32_t)((k / BWD_STAGES) & 1));
-    const int n = min(BWD_CH, cnt - k * BWD_CH);
-    const float4* __restrict__ sA = sm.A[stage];
-    const float4* __restrict__ sC = sm.C[stage];
-    const float2* __restrict__ sB = sm.B[stage] + shift;
-    float* __restrict__ part = sm.partial[warp];
-
-    int j = 0;
-    for (; j < n; ++j) {
-      if ((j & 3) == 0) {
-        bool dead = true;
-#pragma unroll
-        for (int p = 0; p < PX; ++p) dead = dead && !(T[p] > GS_T_STOP);
-        if (__all_sync(0xffffffffu, dead)) break;
-      }
-      const float4 a = sA[j];
-      const float2 b = sB[j];
-      const float4 c = sC[j];
-      float s0 = 0.f, sx = 0.f, sxx = 0.f, c0 = 0.f, c1 = 0.f, c2 = 0.f;
-      const float dy = py - a.y;
-      const float m1 = a.w * dy;
-      const float ev = fmaf(-b.x * dy, dy, b.y);
-#pragma unroll
-      for (int p = 0; p < PX; ++p) {
-        const float dx = px[p] - a.x;
-        const float eu = fmaf(a.z, dx, -m1);
-        const float alpha = gs_ex2(fmaf(-dx, eu, ev));   // l2o - (ca dx^2 - cb dx dy + cc dy^2)
-        const bool live = T[p] > GS_T_STOP;
-        const float w = live ? alpha * T[p] : 0.f;
-        const float gc = fmaf(gr[p], c.x, fmaf(gg[p], c.y, gb[p] * c.z));
-        R[p] = fmaf(-gc, w, R[p]);                                   // sum_c g_c (out_c - C_c^{<=i})
-        const float rc = gs_rcp(1.0000001f - alpha);                 // 1/(1 - alpha + 1e-7)  (:721)
-        const float dal = fmaf(T[p], gc, -R[p] * rc);                // d L / d alpha            (:710-722)
-        const float e = live ? dal * alpha : 0.f;
-        T[p] -= w;
-        const float ex = e * dx;
-        s0 += e;
-        sx += ex;
-        sxx = fmaf(ex, dx, sxx);
-        c0 = fmaf(gr[p], w, c0);
-        c1 = fmaf(gg[p], w, c1);
-        c2 = fmaf(gb[p], w, c2);
-      }
-      float v[8];
-      v[0] = sx;
-      v[1] = dy * s0;
-      v[2] = sxx;
-      v[3] = dy * sx;
-      v[4] = dy * v[1];
-      v[5] = s0;
-      v[6] = c0;
-      v[7] = c1;
-      float v8 = c2;
-      // recursive-halving reduction of v[0..7] over the warp, plain butterfly for v8
-      {
-        const bool up = (lane & 16) != 0;
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const float keep = up ? v[u + 4] : v[u];
-          const float send = up ? v[u] : v[u + 4];
-          v[u] = keep + __shfl_xor_sync(0xffffffffu, send, 16);
-        }
-      }
-      {
-        const bool up = (lane & 8) != 0;
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-          const float keep = up ? v[u + 2] : v[u];
-          const float send = up ? v[u] : v[u + 2];
-          v[u] = keep + __shfl_xor_sync(0xffffffffu, send, 8);
-        }
-      }
-      {
-        const bool up = (lane & 4) != 0;
-        const float keep = up ? v[1] : v[0];
-        const float send = up ? v[0] : v[1];
-        v[0] = keep + __shfl_xor_sync(0xffffffffu, send, 4);
-      }
-      v[0] += __shfl_xor_sync(0xffffffffu, v[0], 2);
-      v[0] += __shfl_xor_sync(0xffffffffu, v[0], 1);
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) v8 += __shfl_xor_sync(0xffffffffu, v8, o);
-      // lane L now holds the warp total of value index ((L>>4)&1)*4 + ((L>>3)&1)*2 + ((L>>2)&1)
-      if ((lane & 3) == 0) part[j * BWD_NV + (((lane >> 4) & 1) * 4 + ((lane >> 3) & 1) * 2 + ((lane >> 2) & 1))] = v[0];
-      if (lane == 0) part[j * BWD_NV + 8] = v8;
-    }
-    // instances this warp skipped because all of its pixels are saturated
-    for (int z = j * BWD_NV + lane; z < n * BWD_NV; z += 32) part[z] = 0.f;
-    __syncthreads();
-
-    for (int t = tid; t < n; t += THREADS) {
-      float s[BWD_NV];
-#pragma unroll
-      for (int u = 0; u < BWD_NV; ++u) {
-        s[u] = sm.partial[0][t * BWD_NV + u];
-#pragma unroll
-        for (int w2 = 1; w2 < WARPS; ++w2) s[u] += sm.partial[w2][t * BWD_NV + u];
-      }
-      const float4 a = sA[t];
-      const float2 b = sB[t];
-      const uint32_t slot = __float_as_uint(sC[t].w);
-      float4* out = reinterpret_cast<float4*>(grad_inst + (size_t)slot * GS_GREC);
-      // d/dx, d/dy, d/dca, d/dcb  |  d/dcc, d/dl2o, d/dr, d/dg  |  d/db
-      out[0] = make_float4(GS_LN2 * (2.f * a.z * s[0] - a.w * s[1]), GS_LN2 * (2.f * b.x * s[1] - a.w * s[0]),
-                           -GS_LN2 * s[2], GS_LN2 * s[3]);
-      out[1] = make_float4(-GS_LN2 * s[4], GS_LN2 * s[5], s[6], s[7]);
-      out[2] = make_float4(s[8], 0.f, 0.f, 0.f);
-      if (row_epoch) row_epoch[slot] = epoch;      // marks the row as written in this frame
-    }
-    bool dead = true;
-#pragma unroll
-    for (int p = 0; p < PX; ++p) dead = dead && !(T[p] > GS_T_STOP);
-    const int all_dead = __syncthreads_and(dead);
-    if (all_dead) {
-      consumed = min(cnt, (k + 1) * BWD_CH);
-      break;
-    }
-    if (tid == 0 && k + BWD_STAGES < nchunks) {
-      const int kn = k + BWD_STAGES;
-      issue_chunk<Smem, BWD_CH>(sm, stage, pA, pB, pC, start + kn * BWD_CH, min(BWD_CH, cnt - kn * BWD_CH), shift);
-    }
-  }
-  if (tid == 0 && k < nchunks) {
-    for (int kk = k + 1; kk < nchunks && kk < k + BWD_STAGES; ++kk)
-      gs_mbar_wait(&sm.full[kk % BWD_STAGES], (uint32_t)((kk / BWD_STAGES) & 1));
-  }
-  if (tile_neff_b && tid == 0) tile_neff_b[tile] = consumed;
-  // the unread tail of a saturated tile has zero gradient: with an epoch array the rows are simply
-  // left stale (the consumer skips rows whose tag is not this frame's); otherwise write zeros
-  if (row_epoch) return;
-  for (int t = consumed + tid; t < cnt; t += THREADS) {
-    const uint32_t slot = __float_as_uint(pC[start + t].w);
-    float4* out = reinterpret_cast<float4*>(grad_inst + (size_t)slot * GS_GREC);
-    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-    out[0] = z;
-    out[1] = z;
-    out[2] = z;
-  }
-}
-
-// =======================================================================================
-// warp-specialised kernels (default): one PRODUCER warp issues the bulk-async copies of the tile's
-// sorted range, chunk by chunk, into a ring of shared-memory stages guarded by full / empty
-// mbarriers; the CONSUMER warps only ever wait on `full`, blend, and release with one arrive on
-// `empty`.  Consumers synchronise among themselves on a named barrier the producer never joins.
-// =======================================================================================
-constexpr int WS_CH = 64;          // instances per staging chunk (40 B each: 2.5 KB per stage)
-
-template <int STAGES>
-struct WsRing {
-  float4 A[STAGES][WS_CH];
-  float4 C[STAGES][WS_CH];
-  float2 B[STAGES][WS_CH + 2];
-  uint64_t full[STAGES], empty[STAGES], done;
-  volatile int stop, consumed_chunks;
-};
-
-template <typename SM, int STAGES>
-__device__ __forceinline__ void ws_init(SM& sm, int tid) {
-  if (tid == 0) {
-    for (int s = 0; s < STAGES; ++s) {
-      gs_mbar_init(&sm.full[s], 1);
-      gs_mbar_init(&sm.empty[s], 1);
-    }
-    gs_mbar_init(&sm.done, 1);
-    sm.stop = 0;
-    sm.consumed_chunks = 0;
-    gs_fence_barrier_init();
-  }
-  __syncthreads();
-}
-
-// Producer warp (one elected lane): keeps up to STAGES chunks in flight; stops as soon as the
-// consumers report that every pixel of the tile is saturated, and drains copies that were issued
-// but never consumed before the CTA may retire (their destination is this CTA's shared memory).
-template <typename SM, int STAGES>
-__device__ __forceinline__ void ws_producer(SM& sm, const float4* __restrict__ pA, const float2* __restrict__ pB,
-                                            const float4* __restrict__ pC, int start, int cnt, int nchunks) {
-  const int shift = start & 1;
-  int k = 0;
-  for (; k < nchunks; ++k) {
-    const int s = k % STAGES;
-    if (k >= STAGES) gs_mbar_wait(&sm.empty[s], (uint32_t)(((k / STAGES) - 1) & 1));
-    if (sm.stop) break;
-    issue_chunk<SM, WS_CH>(sm, s, pA, pB, pC, start + k * WS_CH, min(WS_CH, cnt - k * WS_CH), shift);
-  }
-  gs_mbar_wait(&sm.done, 0u);
-  for (int kk = sm.consumed_chunks; kk < k; ++kk) gs_mbar_wait(&sm.full[kk % STAGES], (uint32_t)((kk / STAGES) & 1));
-}
-
-// ---- forward ---------------------------------------------------------------------------
-constexpr int WSF_STAGES = 4;
-constexpr int WSF_CONS = 64;       // consumer threads: 2 warps, each thread a row of 4 adjacent pixels
-
-__global__ void __launch_bounds__(WSF_CONS + 32) blend_fwd_ws_kernel(const float4* __restrict__ pA,
-                                                                      const float2* __restrict__ pB,
-                                                                      const float4* __restrict__ pC,
-                                                                      const int* __restrict__ tile_accum, int wp,
-                                                                      int hp, int ntx, float fx, float fy,
-                                                                      float* __restrict__ image,
-                                                                      int* __restrict__ tile_neff,
-                                                                      float* __restrict__ final_img, GsCrop crop) {
-  using Smem = WsRing<WSF_STAGES>;
-  __shared__ __align__(16) Smem sm;
-  const int tile = blockIdx.x;
-  const int tid = threadIdx.x;
-  const int start = tile_accum[tile];
-  const int cnt = tile_accum[tile + 1] - start;
-  const int nchunks = (cnt + WS_CH - 1) / WS_CH;
-  ws_init<Smem, WSF_STAGES>(sm, tid);
-  if (tid >= WSF_CONS) {
-    if (tid == WSF_CONS && nchunks > 0) ws_producer<Smem, WSF_STAGES>(sm, pA, pB, pC, start, cnt, nchunks);
-    return;
-  }
-  const int tx = tile % ntx, ty = tile / ntx;
-  const int ix0 = tx * GS_TILE + (tid & 3) * FWD_PX;
-  const int iy = ty * GS_TILE + (tid >> 2);
-  float px[FWD_PX];
-#pragma unroll
-  for (int p = 0; p < FWD_PX; ++p) px[p] = gs_pixel_coord(ix0 + p, wp, fx);
-  const float py = gs_pixel_coord(iy, hp, fy);
-  const int shift = start & 1;
-
-  float T[FWD_PX], cr[FWD_PX], cg[FWD_PX], cb[FWD_PX];
-#pragma unroll
-  for (int p = 0; p < FWD_PX; ++p) {
-    T[p] = 1.f;
-    cr[p] = cg[p] = cb[p] = 0.f;
-  }
-  int consumed = cnt;
-  for (int k = 0; k < nchunks; ++k) {
-    const int stage = k % WSF_STAGES;
-    gs_mbar_wait(&sm.full[stage], (uint32_t)((k / WSF_STAGES) & 1));
-    const int n = min(WS_CH, cnt - k * WS_CH);
-    const float4* __restrict__ sA = sm.A[stage];
-    const float4* __restrict__ sC = sm.C[stage];
-    const float2* __restrict__ sB = sm.B[stage] + shift;
-#define GS_FWD_BODY(J)                                                                      \
-  {                                                                                         \
-    const float4 a = sA[J];                                                                 \
-    const float2 b = sB[J];                                                                 \
-    const float4 c = sC[J];                                                                 \
-    const float dy = py - a.y;                                                              \
-    const float m1 = a.w * dy;                                                              \
-    const float ev = fmaf(-b.x * dy, dy, b.y);                                              \
-    _Pragma("unroll") for (int p = 0; p < FWD_PX; ++p) {                                    \
-      const float dx = px[p] - a.x;                                                         \
-      const float eu = fmaf(a.z, dx, -m1);                                                  \
-      const float alpha = gs_ex2(fmaf(-dx, eu, ev));                                        \
-      const float w = (T[p] > GS_T_STOP) ? alpha * T[p] : 0.f;                              \
-      cr[p] = fmaf(c.x, w, cr[p]);                                                          \
-      cg[p] = fmaf(c.y, w, cg[p]);                                                          \
-      cb[p] = fmaf(c.z, w, cb[p]);                                                          \
-      T[p] -= w;                                                                            \
-    }                                                                                       \
-  }
-    int j = 0;
-    bool warp_dead = false;
-    for (; j + 4 <= n; j += 4) {
-#pragma unroll
-      for (int u = 0; u < 4; ++u) GS_FWD_BODY(j + u)
-      const bool dead = !(T[0] > GS_T_STOP) && !(T[1] > GS_T_STOP) && !(T[2] > GS_T_STOP) && !(T[3] > GS_T_STOP);
-      if (__all_sync(0xffffffffu, dead)) {
-        warp_dead = true;
-        break;
-      }
-    }
-    if (!warp_dead)
-      for (; j < n; ++j) GS_FWD_BODY(j)
-#undef GS_FWD_BODY
-    const bool dead = !(T[0] > GS_T_STOP) && !(T[1] > GS_T_STOP) && !(T[2] > GS_T_STOP) && !(T[3] > GS_T_STOP);
-    const int all_dead = gs_bar_red_and(1, WSF_CONS, dead);       // also: both warps are done with the stage
-    if (all_dead) {
-      consumed = min(cnt, (k + 1) * WS_CH);
-      if (tid == 0) {
-        sm.consumed_chunks = k + 1;
-        sm.stop = 1;
-        gs_mbar_arrive(&sm.empty[stage]);
-      }
-      break;
-    }
-    if (tid == 0) {
-      sm.consumed_chunks = k + 1;
-      gs_mbar_arrive(&sm.empty[stage]);
-    }
-  }
-  if (tid == 0 && nchunks > 0) gs_mbar_arrive(&sm.done);
-  float4* o = reinterpret_cast<float4*>(image + ((size_t)iy * wp + ix0) * 3);
-  o[0] = make_float4(cr[0], cg[0], cb[0], cr[1]);
-  o[1] = make_float4(cg[1], cb[1], cr[2], cg[2]);
-  o[2] = make_float4(cb[2], cr[3], cg[3], cb[3]);
-  if (final_img) {
-#pragma unroll
-    for (int p = 0; p < FWD_PX; ++p)
-      gs_store_final(final_img, ix0 + p, iy, crop.left, crop.top, crop.width, crop.height, cr[p], cg[p], cb[p]);
-  }
-  if (tile_neff && tid == 0) tile_neff[tile] = consumed;
-}
-
-// ---- backward ----------------------------------------------------------------------------
-// Cross-thread reduction WITHOUT shuffles: every consumer thread accumulates, over its own row of
+// Cross-thread reduction WITHOUT shuffles: every thread accumulates, over its own row of
 // PX pixels, six partial sums per instance (S0, Sx, Sxx, Cr, Cg, Cb; dy is shared by the row) and
 // stores them to shared memory ([instance][quarter][thread][6], strides chosen so that both the
 // 8-byte stores and the 8-byte loads of the second phase are bank-conflict free).  After R = NT/4
 // instances a second phase gives each instance to 4 threads: each sums one quarter of the source
 // threads (4 pixel rows: Sy = sum dy S0, Sxy = sum dy Sx, Syy = sum dy^2 S0 are formed per row), two
 // xor-shuffles combine the quarters, and each of the 4 lanes stores one 16-byte piece of the
-// instance's gradient record.  ~13 instructions per (thread, instance) instead of ~42 for the
+// instance's gradient record.  ~13 instructions per (thread, instance) instead of ~42 for a
 // recursive-halving shuffle network; fixed summation order => bit-deterministic.
-template <int PX, int STAGES_, int RQ_, int PW_ = 6>
-struct Bwd2Cfg {
-  static constexpr int NT = 256 / PX;                        // consumer threads (64 or 32)
+constexpr int BWD_PX = 8;                    // each thread owns a row of 8 adjacent pixels
+constexpr int BWD_THREADS = 256 / BWD_PX;    // one warp per tile
+
+// Per-path constants.  gather: the best configuration of the round-2 sweeps (profiles/r2_sweeps.md), 32-instance
+// chunks 3 deep, 4 instances per unrolled step.  packed (legacy draw API, gs_tune("gather", 0)): 64-instance chunks
+// 2 deep, unroll 2.
+template <bool GATHER, bool MAPS>
+struct BwdCfg {
+  static constexpr int PX = BWD_PX, NT = BWD_THREADS;
   static constexpr int TPR = GS_TILE / PX;                   // threads per pixel row
-  static constexpr int RQ = RQ_;                             // reducer threads per instance in the second phase
+  static constexpr int RQ = 4;                               // reducer threads per instance in the second phase
   static constexpr int R = NT / RQ;                          // instances per reduction round
   static constexpr int SQ = NT / RQ;                         // source threads per reducer ("part")
   static constexpr int ROWS = SQ / TPR;                      // pixel rows per reducer
   // floats per (source thread, instance): 6, or 8 for a maps frame - the 7th sum (and a pad) then sits in a
   // [part][source thread][2] block behind the [part][source thread][6] one, so both store streams keep their stride
-  static constexpr int PW = PW_;
+  static constexpr int PW = MAPS ? 8 : 6;
   // strides (floats) of the partial buffer [instance][part][source thread][6 (+2)]: part stride = 32/RQ and
   // instance stride = 2 (mod 32) make the 8-byte loads of a half-warp (16 / RQ instances x RQ parts) hit
   // 16 distinct bank pairs; the 8-byte stores of 16 consecutive source threads (stride 6, resp. 2) are conflict free
   static constexpr int QS = (SQ * PW + 31) / 32 * 32 + 32 / RQ;
   static constexpr int IS = RQ * QS + 2 - (RQ * QS) % 32 + ((RQ * QS) % 32 > 2 ? 32 : 0);
-  static constexpr int STAGES = STAGES_;
+  static constexpr int CH = GATHER ? 32 : 64;                // instances per staging chunk
+  static constexpr int STAGES = GATHER ? 3 : 2;              // staging ring depth
+  static constexpr int UNR = GATHER ? 4 : 2;                 // instances per unrolled step of the first phase
+  static constexpr int MINB = GATHER ? 10 : 16;              // __launch_bounds__ min blocks (register cap)
 };
 
-template <int PX, int STAGES, int RQ, bool GATHER, int CH, int PW = 6>
-struct Bwd2Smem : std::conditional<GATHER, GatherRing<CH, STAGES, 4>, WsRing<STAGES>>::type {
-  float part[Bwd2Cfg<PX, STAGES, RQ, PW>::R * Bwd2Cfg<PX, STAGES, RQ, PW>::IS];
+template <bool GATHER, bool MAPS>
+struct BwdSmem : std::conditional<GATHER, GatherRing<BwdCfg<GATHER, MAPS>::CH, BwdCfg<GATHER, MAPS>::STAGES, 4>,
+                                  PackedRing<BwdCfg<GATHER, MAPS>::CH, BwdCfg<GATHER, MAPS>::STAGES>>::type {
+  float part[BwdCfg<GATHER, MAPS>::R * BwdCfg<GATHER, MAPS>::IS];
   float pyt[GS_TILE];
-  int valid[2];
 };
 
 // Upstream gradients of the depth and alpha maps for a thread's row of PX pixels (MAPS only)
@@ -811,30 +425,27 @@ __device__ __forceinline__ void bwd_row(const float4 a, const float2 b, const fl
   if constexpr (MAPS) dst_d[0] = make_float2(cd, 0.f);
 }
 
-// WS: dedicated producer warp (full / empty mbarrier ring); !WS: consumer thread 0 issues the copies at the
-// chunk boundaries (no extra warp holding registers).  UNR: instances per unrolled step of the first phase.
+// Thread 0 (packed) or every thread (gather) issues the copies of the next chunk at the chunk boundaries.
 // MAPS (gather path only): gradients of the depth / alpha maps too; d/d depth_i goes to float 9 of the gradient row.
-// `maps` is the last parameter so that the other instantiations keep their parameter offsets (and their code).
-template <int PX, bool WS, int UNR, int STAGES, int MINB, int RQ, bool GATHER, int CH, bool MAPS = false>
-__global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
-    blend_bwd2_kernel(const float4* __restrict__ pA, const float2* __restrict__ pB, const float4* __restrict__ pC,
-                      const GsRec* __restrict__ grec, const uint32_t* __restrict__ ids,
-                      const uint32_t* __restrict__ goff, const int* __restrict__ tile_accum, int wp, int hp, int ntx, float fx, float fy,
-                      const float* __restrict__ image, const float* __restrict__ grad_image,
-                      float* __restrict__ grad_inst, int grad_is_final, GsCrop crop, uint32_t* __restrict__ row_epoch,
-                      uint32_t epoch, int* __restrict__ tile_neff_b, GsMapsBwd maps = GsMapsBwd{}) {
-  constexpr int PW = MAPS ? 8 : 6;
-  using Cfg = Bwd2Cfg<PX, STAGES, RQ, PW>;
-  constexpr int NT = Cfg::NT, TPR = Cfg::TPR, R = Cfg::R, SQ = Cfg::SQ, QS = Cfg::QS, IS = Cfg::IS, ROWS = Cfg::ROWS;
+template <bool GATHER, bool MAPS>
+__global__ void __launch_bounds__(BWD_THREADS, BwdCfg<GATHER, MAPS>::MINB)
+    blend_bwd_kernel(const float4* __restrict__ pA, const float2* __restrict__ pB, const float4* __restrict__ pC,
+                     const GsRec* __restrict__ grec, const uint32_t* __restrict__ ids,
+                     const uint32_t* __restrict__ goff, const int* __restrict__ tile_accum, int wp, int hp, int ntx, float fx, float fy,
+                     const float* __restrict__ image, const float* __restrict__ grad_image,
+                     float* __restrict__ grad_inst, int grad_is_final, GsCrop crop, uint32_t* __restrict__ row_epoch,
+                     uint32_t epoch, int* __restrict__ tile_neff_b, GsMapsBwd maps) {
+  using Cfg = BwdCfg<GATHER, MAPS>;
+  constexpr int PX = Cfg::PX, NT = Cfg::NT, TPR = Cfg::TPR, RQ = Cfg::RQ, R = Cfg::R, SQ = Cfg::SQ, QS = Cfg::QS,
+                IS = Cfg::IS, ROWS = Cfg::ROWS, CH = Cfg::CH, STAGES = Cfg::STAGES, UNR = Cfg::UNR;
   static_assert(IS % 2 == 0 && QS % 2 == 0 && IS % 32 == 2 && QS % 32 == 32 / RQ, "partial buffer strides");
-  static_assert(!(WS && GATHER), "the gather path issues its copies from all consumer threads");
-  static_assert(GATHER || CH == WS_CH, "the packed ring is sized for CH instances per stage");
+  static_assert(NT == 32, "one warp per tile: warp votes and __syncwarp order the phases");
   static_assert(!MAPS || GATHER, "depth / alpha maps read the depth from the gathered records");
   static_assert(PX % 4 == 0, "float4 rows of the image / map planes");
-  using Smem = Bwd2Smem<PX, STAGES, RQ, GATHER, CH, PW>;
+  using Smem = BwdSmem<GATHER, MAPS>;
   __shared__ __align__(16) Smem sm;
   const int tile = blockIdx.x;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int tid = threadIdx.x;
   const int start = tile_accum[tile];
   const int cnt = tile_accum[tile + 1] - start;
   if (cnt == 0) return;
@@ -842,24 +453,11 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
   const int tx = tile % ntx, ty = tile / ntx;
   const int shift = start & 1;
   if (tid < GS_TILE) sm.pyt[tid] = gs_pixel_coord(ty * GS_TILE + tid, hp, fy);
-  if constexpr (GATHER) {
-    if (tid == 0) {
-      for (int s = 0; s < STAGES; ++s) gs_mbar_init(&sm.full[s], NT);
-      gs_fence_barrier_init();
-    }
-    __syncthreads();
-  } else {
-    ws_init<Smem, STAGES>(sm, tid);
-    if (WS) {
-      if (tid >= NT) {
-        if (tid == NT) ws_producer<Smem, STAGES>(sm, pA, pB, pC, start, cnt, nchunks);
-        return;
-      }
-    } else if (tid == 0) {
-      for (int k = 0; k < STAGES && k < nchunks; ++k)
-        issue_chunk<Smem, CH>(sm, k, pA, pB, pC, start + k * CH, min(CH, cnt - k * CH), shift);
-    }
+  if (tid == 0) {
+    for (int s = 0; s < STAGES; ++s) gs_mbar_init(&sm.full[s], GATHER ? NT : 1);
+    gs_fence_barrier_init();
   }
+  __syncthreads();
   GatherIds<NT, CH> gid;
   if constexpr (GATHER) {
     for (int k = 0; k < STAGES && k < nchunks; ++k) {
@@ -867,6 +465,9 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
       gather_issue<Smem, NT, CH, 4>(sm, k, grec, goff, gid, min(CH, cnt - k * CH), tid);
     }
     if (STAGES < nchunks) gid.load(ids, start + STAGES * CH, min(CH, cnt - STAGES * CH), tid);
+  } else if (tid == 0) {
+    for (int k = 0; k < STAGES && k < nchunks; ++k)
+      issue_chunk<Smem>(sm, k, pA, pB, pC, start + k * CH, min(CH, cnt - k * CH), shift);
   }
   const int ix0 = tx * GS_TILE + (tid % TPR) * PX;
   const int iy = ty * GS_TILE + (tid / TPR);
@@ -986,25 +587,15 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
                             my_part + (j + u) * (IS / 2), MAPS ? sv.depth(sub + j + u) : 0.f, &mg,
                             my_part_d + (j + u) * (IS / 2));
       }
-      if (UNR > 1 && !wdead)
+      if (!wdead)
         for (; j < nr; ++j)
           bwd_row<PX, MAPS>(sv.a(sub + j), sv.b(sub + j), sv.c(sub + j), px, py, T, Rr, gr, gg, gb,
                             my_part + j * (IS / 2), MAPS ? sv.depth(sub + j) : 0.f, &mg, my_part_d + j * (IS / 2));
       bool dead = true;
 #pragma unroll
       for (int p = 0; p < PX; ++p) dead = dead && !(T[p] > GS_T_STOP);
-      int all_dead;
-      int v0, v1;
-      if (NT == 64) {
-        if (lane == 0) sm.valid[warp] = j;          // j is warp-uniform (the loop only breaks on a warp vote)
-        all_dead = gs_bar_red_and(1, NT, dead);
-        v0 = sm.valid[0];
-        v1 = sm.valid[1];
-      } else {
-        __syncwarp();
-        all_dead = __all_sync(0xffffffffu, dead);
-        v0 = v1 = j;
-      }
+      __syncwarp();
+      const int all_dead = __all_sync(0xffffffffu, dead);
       // ---- phase 2: 4 threads per instance, one quarter of the source threads (4 pixel rows) each
       {
         float S0 = 0.f, Sx = 0.f, Sxx = 0.f, Sy = 0.f, Sxy = 0.f, Syy = 0.f, C0 = 0.f, C1 = 0.f, C2 = 0.f, Cd = 0.f;
@@ -1015,8 +606,7 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
           a = sv.a(sub + ri);
           b = sv.b(sub + ri);
         }
-        const int vq = (NT == 64 && rq * SQ >= 32) ? v1 : v0;   // instances the part's source warp really processed
-        if (act && ri < vq) {
+        if (act && ri < j) {                       // j: instances the warp really processed (warp-uniform)
 #pragma unroll
           for (int r = 0; r < ROWS; ++r) {
             float2 u0 = red_src[(r * TPR) * 3], u1 = red_src[(r * TPR) * 3 + 1], u2 = red_src[(r * TPR) * 3 + 2];
@@ -1046,8 +636,7 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
         }
 #define GS_RED4(V)                                   \
   V += __shfl_xor_sync(0xffffffffu, V, 1);           \
-  V += __shfl_xor_sync(0xffffffffu, V, 2);           \
-  if (RQ == 8) V += __shfl_xor_sync(0xffffffffu, V, 4);
+  V += __shfl_xor_sync(0xffffffffu, V, 2);
         GS_RED4(S0) GS_RED4(Sx) GS_RED4(Sxx) GS_RED4(Sy) GS_RED4(Sxy) GS_RED4(Syy) GS_RED4(C0) GS_RED4(C1) GS_RED4(C2)
         if constexpr (MAPS) { GS_RED4(Cd) }
 #undef GS_RED4
@@ -1066,8 +655,7 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
             row_epoch[slot] = epoch;               // marks the row as written in this frame
         }
       }
-      if (NT == 64) gs_bar_sync(1, NT);            // the partial buffer may be overwritten now
-      else __syncwarp();
+      __syncwarp();                               // the partial buffer may be overwritten now
       if (all_dead) {
         consumed = min(cnt, k * CH + sub + nr);
         finished = true;
@@ -1075,26 +663,18 @@ __global__ void __launch_bounds__(256 / PX + (WS ? 32 : 0), MINB)
       }
     }
     if constexpr (GATHER) {
-      if (!finished && k + STAGES < nchunks) {   // every consumer is past the barrier: the stage is free
+      if (!finished && k + STAGES < nchunks) {   // every thread is past the barrier: the stage is free
         const int kn = k + STAGES;
         gather_issue<Smem, NT, CH, 4>(sm, stage, grec, goff, gid, min(CH, cnt - kn * CH), tid);
         if (kn + 1 < nchunks) gid.load(ids, start + (kn + 1) * CH, min(CH, cnt - (kn + 1) * CH), tid);
       }
-    } else if (tid == 0) {
-      if (WS) {
-        sm.consumed_chunks = k + 1;
-        if (finished) sm.stop = 1;
-        gs_mbar_arrive(&sm.empty[stage]);
-      } else if (!finished && k + STAGES < nchunks) {
-        const int kn = k + STAGES;               // every consumer is past the barrier: the stage is free
-        issue_chunk<Smem, CH>(sm, stage, pA, pB, pC, start + kn * CH, min(CH, cnt - kn * CH), shift);
-      }
+    } else if (tid == 0 && !finished && k + STAGES < nchunks) {
+      const int kn = k + STAGES;                 // every thread is past the barrier: the stage is free
+      issue_chunk<Smem>(sm, stage, pA, pB, pC, start + kn * CH, min(CH, cnt - kn * CH), shift);
     }
   }
   if (tid == 0) {
-    if constexpr (!GATHER && WS) {
-      gs_mbar_arrive(&sm.done);
-    } else if (finished) {
+    if (finished) {
       // drain copies that were issued but never consumed before the CTA may retire (k was incremented past the
       // chunk that finished): chunks k .. k + STAGES - 2 are in flight
       for (int kk = k; kk < nchunks && kk < k + STAGES - 1; ++kk)
@@ -1234,28 +814,9 @@ inline size_t legacy_ws_layout(int m, int d, LegacyWs* ws, char* base) {
 cudaError_t gs_launch_blend_fwd(const float4* pA, const float2* pB, const float4* pC, const GsRec* grec,
                                 const uint32_t* ids, const int* tile_accum, const GsFrameGeom& g, float* image,
                                 int* tile_neff, float* final_img, const GsCrop& crop, cudaStream_t st) {
-  const GsTuning& tn = gs_tuning();
-  const bool gather = grec != nullptr;
-  if (!gather && tn.fwd_kernel != 0) {
-    blend_fwd_ws_kernel<<<g.n_tiles, WSF_CONS + 32, 0, st>>>(pA, pB, pC, tile_accum, g.wp, g.hp, g.ntx, g.fx, g.fy, image,
-                                                             tile_neff, final_img, crop);
-    return cudaGetLastError();
-  }
-  const int ch = tn.fwd_ch;   // staging chunk
-#define GS_FWD_LAUNCH(CH, PX, GA)                                                                                   \
-  blend_fwd_kernel<CH, PX, GA><<<g.n_tiles, 256 / PX, 0, st>>>(pA, pB, pC, grec, ids, tile_accum, g.wp, g.hp, g.ntx, \
-                                                               g.fx, g.fy, image, tile_neff, final_img, crop)
-#define GS_FWD_CH(PX, GA)                     \
-  if (ch == 64) GS_FWD_LAUNCH(64, PX, GA);    \
-  else if (ch == 256) GS_FWD_LAUNCH(256, PX, GA); \
-  else GS_FWD_LAUNCH(128, PX, GA)
-  if (gather) {
-    if (tn.fwd_px == 8) { GS_FWD_CH(8, true); } else { GS_FWD_CH(4, true); }
-  } else {
-    if (tn.fwd_px == 8) { GS_FWD_CH(8, false); } else { GS_FWD_CH(4, false); }
-  }
-#undef GS_FWD_CH
-#undef GS_FWD_LAUNCH
+  const auto kernel = grec ? blend_fwd_kernel<true, false> : blend_fwd_kernel<false, false>;
+  kernel<<<g.n_tiles, FWD_THREADS, 0, st>>>(pA, pB, pC, grec, ids, tile_accum, g.wp, g.hp, g.ntx, g.fx, g.fy, image,
+                                            tile_neff, final_img, crop, GsMapsFwd{});
   return cudaGetLastError();
 }
 
@@ -1264,88 +825,14 @@ cudaError_t gs_launch_blend_bwd(const float4* pA, const float2* pB, const float4
                                 const float* image,
                                 const float* grad_image, float* grad_inst, int grad_is_final, const GsCrop& crop,
                                 uint32_t* row_epoch, uint32_t epoch, int* tile_neff_b, cudaStream_t st) {
-  const GsTuning& tn = gs_tuning();
-  const bool gather = grec != nullptr;
-  if (gather && !row_epoch) return cudaErrorInvalidValue;
-  if (tn.bwd_kernel != 0 || gather) {
-#define GS_BWD2C(PX, WS, UNR, ST, MINB, RQ, GA, CH)                                                                 \
-  blend_bwd2_kernel<PX, WS, UNR, ST, MINB, RQ, GA, CH><<<g.n_tiles, 256 / PX + (WS ? 32 : 0), 0, st>>>(              \
-      pA, pB, pC, grec, ids, goff, tile_accum, g.wp, g.hp, g.ntx, g.fx, g.fy, image, grad_image, grad_inst,          \
-      grad_is_final,                                                                                                 \
-      crop, row_epoch, epoch, tile_neff_b)
-#define GS_BWD2(PX, WS, UNR, ST, MINB, RQ, GA) GS_BWD2C(PX, WS, UNR, ST, MINB, RQ, GA, 64)
-    // key: px | producer warp | unroll | stages | reducers per instance | min blocks (2 digits)
-    const int key = ((((tn.bwd_px * 10 + tn.bwd_ws) * 10 + tn.bwd_unroll) * 10 + tn.bwd_stages) * 10 + tn.bwd_rq) * 100 +
-                    tn.bwd_minb;
-    if (gather && tn.bwd_ch == 32) {
-      switch (key) {
-        case 8022416: GS_BWD2C(8, false, 2, 2, 16, 4, true, 32); break;
-        case 8023416: GS_BWD2C(8, false, 2, 3, 16, 4, true, 32); break;
-        case 8042410: GS_BWD2C(8, false, 4, 2, 10, 4, true, 32); break;
-        case 8043410: GS_BWD2C(8, false, 4, 3, 10, 4, true, 32); break;
-        default: return gs_tuning().strict ? cudaErrorInvalidValue : (GS_BWD2C(8, false, 4, 3, 10, 4, true, 32), cudaGetLastError());
-      }
-      return cudaGetLastError();
-    }
-    if (gather) {
-      switch (key) {
-        case 8012410: GS_BWD2(8, false, 1, 2, 10, 4, true); break;
-        case 8022416: GS_BWD2(8, false, 2, 2, 16, 4, true); break;
-        case 8022410: GS_BWD2(8, false, 2, 2, 10, 4, true); break;
-        case 8042410: GS_BWD2(8, false, 4, 2, 10, 4, true); break;
-        case 8023416: GS_BWD2(8, false, 2, 3, 16, 4, true); break;
-        case 8012416: GS_BWD2(8, false, 1, 2, 16, 4, true); break;
-        case 8012420: GS_BWD2(8, false, 1, 2, 20, 4, true); break;
-        case 8012820: GS_BWD2(8, false, 1, 2, 20, 8, true); break;
-        case 8013416: GS_BWD2(8, false, 1, 3, 16, 4, true); break;
-        case 4012401: GS_BWD2(4, false, 1, 2, 1, 4, true); break;
-        case 4042401: GS_BWD2(4, false, 4, 2, 1, 4, true); break;
-        default: return gs_tuning().strict ? cudaErrorInvalidValue : (GS_BWD2(8, false, 2, 2, 16, 4, true), cudaGetLastError());
-      }
-      return cudaGetLastError();
-    }
-    switch (key) {
-      case 4113401: GS_BWD2(4, true, 1, 3, 1, 4, false); break;      // round-2 first version
-      case 4143408: GS_BWD2(4, true, 4, 3, 8, 4, false); break;
-      case 4012401: GS_BWD2(4, false, 1, 2, 1, 4, false); break;
-      case 4042401: GS_BWD2(4, false, 4, 2, 1, 4, false); break;
-      case 4042810: GS_BWD2(4, false, 4, 2, 10, 8, false); break;
-      case 8012410: GS_BWD2(8, false, 1, 2, 10, 4, false); break;
-      case 8012416: GS_BWD2(8, false, 1, 2, 16, 4, false); break;
-      case 8012420: GS_BWD2(8, false, 1, 2, 20, 4, false); break;
-      case 8013416: GS_BWD2(8, false, 1, 3, 16, 4, false); break;
-      case 8022416: GS_BWD2(8, false, 2, 2, 16, 4, false); break;
-      case 8022410: GS_BWD2(8, false, 2, 2, 10, 4, false); break;
-      case 8042410: GS_BWD2(8, false, 4, 2, 10, 4, false); break;
-      case 8012816: GS_BWD2(8, false, 1, 2, 16, 8, false); break;
-      case 8012820: GS_BWD2(8, false, 1, 2, 20, 8, false); break;
-      case 8112410: GS_BWD2(8, true, 1, 2, 10, 4, false); break;
-      case 8012424: GS_BWD2(8, false, 1, 2, 24, 4, false); break;
-      case 8012824: GS_BWD2(8, false, 1, 2, 24, 8, false); break;
-      // the packed path (legacy draw API, gs_tune("gather", 0)) has fewer instantiated variants than the gather
-      // path: any other knob combination runs its shipped configuration (strict mode, used by the sweeps, refuses)
-      default: return gs_tuning().strict ? cudaErrorInvalidValue : (GS_BWD2(8, false, 2, 2, 16, 4, false), cudaGetLastError());
-    }
-#undef GS_BWD2
-#undef GS_BWD2C
-    return cudaGetLastError();
-  }
-  const int warps = tn.bwd_px == 8 ? 1 : 2;   // round-1 kernel: 1 warp x 8 px or 2 warps x 4 px
-  const int ch = 64;
-#define GS_BWD_LAUNCH(W, CH)                                                                                         \
-  blend_bwd_kernel<W, CH><<<g.n_tiles, 32 * W, 0, st>>>(pA, pB, pC, tile_accum, g.wp, g.hp, g.ntx, g.fx, g.fy, image, \
-                                                        grad_image, grad_inst, grad_is_final, crop, row_epoch, epoch, \
-                                                        tile_neff_b)
-  if (warps == 1) GS_BWD_LAUNCH(1, 64);
-  else if (ch == 32) GS_BWD_LAUNCH(2, 32);
-  else if (ch == 128) GS_BWD_LAUNCH(2, 128);
-  else GS_BWD_LAUNCH(2, 64);
-#undef GS_BWD_LAUNCH
+  if (grec && !row_epoch) return cudaErrorInvalidValue;
+  const auto kernel = grec ? blend_bwd_kernel<true, false> : blend_bwd_kernel<false, false>;
+  kernel<<<g.n_tiles, BWD_THREADS, 0, st>>>(pA, pB, pC, grec, ids, goff, tile_accum, g.wp, g.hp, g.ntx, g.fx, g.fy, image,
+                                            grad_image, grad_inst, grad_is_final, crop, row_epoch, epoch, tile_neff_b,
+                                            GsMapsBwd{});
   return cudaGetLastError();
 }
 
-// Maps frames always run the shipped gather configurations (forward: 128-instance chunks, 4 pixels per thread;
-// backward: 8 pixels per thread, 4-instance unroll, 3 stages, MINB 10, 4 reducers, 32-instance chunks).
 cudaError_t gs_launch_blend_fwd_maps(const GsRec* grec, const uint32_t* ids, const int* tile_accum, const GsFrameGeom& g,
                                      float* image, int* tile_neff, float* final_img, const GsCrop& crop,
                                      const GsMapsFwd& maps, cudaStream_t st) {
@@ -1354,9 +841,9 @@ cudaError_t gs_launch_blend_fwd_maps(const GsRec* grec, const uint32_t* ids, con
   if (!maps.depth || !maps.alpha || (final_img != nullptr) != (maps.depth_final != nullptr) ||
       (maps.depth_final != nullptr) != (maps.alpha_final != nullptr))
     return cudaErrorInvalidValue;
-  blend_fwd_kernel<128, 4, true, true><<<g.n_tiles, 64, 0, st>>>(nullptr, nullptr, nullptr, grec, ids, tile_accum, g.wp,
-                                                                 g.hp, g.ntx, g.fx, g.fy, image, tile_neff, final_img,
-                                                                 crop, maps);
+  blend_fwd_kernel<true, true><<<g.n_tiles, FWD_THREADS, 0, st>>>(nullptr, nullptr, nullptr, grec, ids, tile_accum, g.wp,
+                                                                   g.hp, g.ntx, g.fx, g.fy, image, tile_neff, final_img,
+                                                                   crop, maps);
   return cudaGetLastError();
 }
 
@@ -1367,9 +854,10 @@ cudaError_t gs_launch_blend_bwd_maps(const GsRec* grec, const uint32_t* ids, con
   // only launched for frames with tile instances (an empty frame has no blend backward), so the records exist
   if (!grec || !ids || !goff || !row_epoch || !maps.depth || !maps.alpha || !maps.grad_depth || !maps.grad_alpha)
     return cudaErrorInvalidValue;
-  blend_bwd2_kernel<8, false, 4, 3, 10, 4, true, 32, true><<<g.n_tiles, 32, 0, st>>>(
-      nullptr, nullptr, nullptr, grec, ids, goff, tile_accum, g.wp, g.hp, g.ntx, g.fx, g.fy, image, grad_image,
-      grad_inst, grad_is_final, crop, row_epoch, epoch, tile_neff_b, maps);
+  blend_bwd_kernel<true, true><<<g.n_tiles, BWD_THREADS, 0, st>>>(nullptr, nullptr, nullptr, grec, ids, goff, tile_accum,
+                                                                  g.wp, g.hp, g.ntx, g.fx, g.fy, image, grad_image,
+                                                                  grad_inst, grad_is_final, crop, row_epoch, epoch,
+                                                                  tile_neff_b, maps);
   return cudaGetLastError();
 }
 

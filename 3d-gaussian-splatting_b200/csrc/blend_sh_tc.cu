@@ -39,12 +39,12 @@ struct TcStage {
   uint64_t full[STAGES];
 };
 
-// NT / 16 threads per instance: record (3 x 16 B), first gradient row (backward), raw coefficients
-template <int K, int STAGES, bool BWD, int NT = TC_NT>
+// TC_NT / 16 threads per instance: record (3 x 16 B), first gradient row (backward), raw coefficients
+template <int K, int STAGES, bool BWD>
 __device__ __forceinline__ void tc_gather(TcStage<K, STAGES>& sm, int stage, const GsRec* __restrict__ grec,
                                           const float* __restrict__ rgb, const uint32_t* __restrict__ ids,
                                           const uint32_t* __restrict__ goff, int base, int n, int tid) {
-  constexpr int SW = sh_sw(K), D = 3 * K, TPI = NT / TC_J;   // threads per instance
+  constexpr int SW = sh_sw(K), D = 3 * K, TPI = TC_NT / TC_J;   // threads per instance
   static_assert(TPI >= 4, "the record pieces and the row offset need four threads");
   const int i = tid / TPI, l = tid % TPI;
   if (i < n) {
@@ -589,297 +589,6 @@ __global__ void __launch_bounds__(TC_NT) blend_sh_bwd_tc_kernel(const GsRec* __r
   if (tile_neff_b && tid == 0) tile_neff_b[tile] = consumed;
 }
 
-
-// ---------------------------------------------------------------------------------------
-// backward, TWO pixels per thread: 128 threads per tile, thread t owns pixels t (accumulator block 0) and t + 128
-// (block 1: same column, 8 rows below) - both in TMEM lane t.  The per-instance work that one pixel per thread
-// repeats for every 32 pixels (record loads, dx, the shuffle reduction of the six geometry sums) is shared by
-// 64 pixels, and every thread carries two independent blend recurrences.  Same operands, schedule and
-// result rows as blend_sh_bwd_tc_kernel.
-// ---------------------------------------------------------------------------------------
-template <int K>
-__global__ void __launch_bounds__(128) blend_sh_bwd_tc2_kernel(const GsRec* __restrict__ grec, const float* __restrict__ rgb,
-                                                               const uint32_t* __restrict__ ids,
-                                                               const uint32_t* __restrict__ goff,
-                                                               const int* __restrict__ tile_accum, int wp, int hp, int ntx,
-                                                               float fx, float fy, const float* __restrict__ rays_o,
-                                                               const float* __restrict__ lefttop,
-                                                               const float* __restrict__ vdx, const float* __restrict__ vdy,
-                                                               const float* __restrict__ image,
-                                                               const float* __restrict__ grad_image,
-                                                               float* __restrict__ grad_inst, int grad_is_final, GsCrop crop,
-                                                               uint32_t* __restrict__ row_epoch, uint32_t epoch,
-                                                               int* __restrict__ tile_neff_b) {
-  constexpr int NT = 128, STAGES = 4, TCOLS = 256, NV = sh_nv(K), GREC = (NV + 3) / 4 * 4;
-  constexpr uint32_t D2COL = 96;
-  extern __shared__ __align__(128) uint8_t tc_smem_raw[];
-  TcBwdSmem<K>& sm = *reinterpret_cast<TcBwdSmem<K>*>(tc_smem_raw);
-  const int tile = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int tx = tile % ntx, ty = tile / ntx;
-  const int ix = tx * GS_TILE + (tid & 15), iy0 = ty * GS_TILE + (tid >> 4), iy1 = iy0 + 8;
-  const int start = tile_accum[tile];
-  const int cnt = tile_accum[tile + 1] - start;
-  if (cnt == 0) return;
-  const int nchunks = (cnt + TC_J - 1) / TC_J;
-  if (tid == 0) {
-    for (int s = 0; s < STAGES; ++s) gs_mbar_init(&sm.st.full[s], NT);
-    gs_mbar_init(&sm.mma_bar, 1);
-    gs_mbar_init(&sm.mma2_bar, 1);
-    gs_fence_barrier_init();
-  }
-  if (warp == 0) tmem_alloc<TCOLS>(&sm.tmem_base);
-  {
-    float sh[16];
-    pixel_sh<K>(ix, iy0, rays_o, lefttop, vdx, vdy, sh);
-    tc_store_basis<K>(sh, sm.img_hi, sm.img_lo, tid);
-    pixel_sh<K>(ix, iy1, rays_o, lefttop, vdx, vdy, sh);
-    tc_store_basis<K>(sh, sm.img_hi, sm.img_lo, tid + 128);
-  }
-  if (tid < 96) {
-    sm.bc_hi[tid] = make_uint4(0, 0, 0, 0);
-    sm.bc_lo[tid] = make_uint4(0, 0, 0, 0);
-  }
-  float T[2] = {1.f, 1.f}, R[2], gr[2], gg[2], gb[2];
-#pragma unroll
-  for (int p = 0; p < 2; ++p) {
-    const int iy = p ? iy1 : iy0;
-    const size_t off = ((size_t)iy * wp + ix) * 3;
-    const float raw[3] = {image[off], image[off + 1], image[off + 2]};
-    if (!grad_is_final) {
-      gr[p] = grad_image[off];
-      gg[p] = grad_image[off + 1];
-      gb[p] = grad_image[off + 2];
-    } else {
-      gs_load_final_grad(grad_image, raw, ix, iy, crop.left, crop.top, crop.width, crop.height, gr[p], gg[p], gb[p]);
-    }
-    R[p] = gr[p] * raw[0] + gg[p] * raw[1] + gb[p] * raw[2];
-  }
-  fence_before_sync();
-  __syncthreads();
-  fence_after_sync();
-  const uint32_t tm = sm.tmem_base;
-  const uint32_t tlane = (uint32_t)(warp * 32) << 16;
-  const uint32_t trow = tm + tlane;                         // block b: + 48 b
-  const float px = gs_pixel_coord(ix, wp, fx);
-  const float py[2] = {gs_pixel_coord(iy0, hp, fy), gs_pixel_coord(iy1, hp, fy)};
-  for (int k = 0; k < STAGES - 1 && k < nchunks; ++k)
-    tc_gather<K, STAGES, true, NT>(sm.st, k, grec, rgb, ids, goff, start + k * TC_J, min(TC_J, cnt - k * TC_J), tid);
-
-  // (np, Rp: instance count and staged records of THAT round - its stage is not refilled before the next barrier)
-  auto epilogue = [&](int np, const float4* Rp) {
-    if (warp < 3) {
-      float a[32], b[32];
-      tmem_ld32(tm + tlane + D2COL, a);
-      tmem_ld32(tm + tlane + D2COL + 32, b);
-      if (tid >= 48) {
-#pragma unroll
-        for (int q = 0; q < 16; ++q) sm.epi[tid - 48][q] = a[q] + b[q];
-      }
-      gs_bar_sync(1, 96);
-      if (tid < 48) {
-        const int c = tid >> 4, j = tid & 15;
-        if (j < np) {
-          const float4 cc = Rp[4 * j + 2];
-          const uint32_t rxy = __float_as_uint(cc.z), rwh = __float_as_uint(cc.w);
-          const uint32_t slot = __float_as_uint(Rp[4 * j + 3].x) + ((uint32_t)ty - (rxy >> 16)) * (rwh & 0xffffu) +
-                                ((uint32_t)tx - (rxy & 0xffffu));
-          float* out = grad_inst + (size_t)slot * GREC + 6 + c * K;
-#pragma unroll
-          for (int q = 0; q < K; ++q) out[q] = ((a[q] + b[q]) + (a[16 + q] + b[16 + q])) + sm.epi[tid][q];
-        }
-      }
-    }
-  };
-
-  // one instance, both pixels: blend state updates, logit gradients dc[pixel][3], summed geometry values v[0..7]
-  auto pair2 = [&](const float4 a, const float4 b4, const float* l0, const float* l1, float (*dc)[3], float* v) {
-    const float dx = px - a.x;
-    const float adx = a.z * dx;
-    float e2[2], ey2[2];
-#pragma unroll
-    for (int p = 0; p < 2; ++p) {
-      const float dy = py[p] - a.y;
-      const float eu = fmaf(-a.w, dy, adx);
-      const float ev = fmaf(-b4.x * dy, dy, b4.y);
-      const float alpha = gs_ex2(fmaf(-dx, eu, ev));
-      const bool live = T[p] > GS_T_STOP;
-      const float w = live ? alpha * T[p] : 0.f;
-      float col[3];
-      const float* l = p ? l1 : l0;
-      tc_colours(l[0], l[1], l[2], col);
-      const float gc = fmaf(gr[p], col[0], fmaf(gg[p], col[1], gb[p] * col[2]));
-      R[p] = fmaf(-gc, w, R[p]);
-      const float rc = gs_rcp(1.0000001f - alpha);
-      const float dal = fmaf(T[p], gc, -R[p] * rc);
-      const float e = live ? dal * alpha : 0.f;
-      T[p] -= w;
-      e2[p] = e;
-      ey2[p] = e * dy;
-      v[4] = p ? fmaf(ey2[1], dy, v[4]) : ey2[0] * dy;
-      dc[p][0] = gr[p] * w * col[0] * (1.f - col[0]);
-      dc[p][1] = gg[p] * w * col[1] * (1.f - col[1]);
-      dc[p][2] = gb[p] * w * col[2] * (1.f - col[2]);
-    }
-    const float es = e2[0] + e2[1], eys = ey2[0] + ey2[1];
-    const float ex = es * dx;
-    v[0] = ex;
-    v[1] = eys;
-    v[2] = ex * dx;
-    v[3] = eys * dx;
-    v[5] = es;
-    v[6] = 0.f;
-    v[7] = 0.f;
-  };
-
-  int consumed = cnt, n_prev = 0, st_prev = 0;
-  uint32_t par_prev = 0;
-  gs_mbar_wait(&sm.st.full[0], 0);
-  tc_split_coefs<K>(sm.st.S[0], sm.bc_hi, sm.bc_lo, tid);
-  fence_smem_to_async();
-  fence_before_sync();
-  __syncthreads();
-  if (warp == 0) {
-    if (elect_one()) {
-      fence_after_sync();
-      tc_issue_logits(tm, sm.img_hi, sm.img_lo, sm.bc_hi, sm.bc_lo, &sm.mma_bar);
-    }
-    __syncwarp();
-  }
-  for (int k = 0; k < nchunks; ++k) {
-    const int stage = k % STAGES;
-    const int n = min(TC_J, cnt - k * TC_J);
-    gs_mbar_wait(&sm.st.full[stage], (uint32_t)((k / STAGES) & 1));
-    gs_mbar_wait(&sm.mma_bar, (uint32_t)(k & 1));
-    fence_after_sync();
-    if (k + 1 < nchunks) {
-      gs_mbar_wait(&sm.st.full[(k + 1) % STAGES], (uint32_t)(((k + 1) / STAGES) & 1));
-      tc_split_coefs<K>(sm.st.S[(k + 1) % STAGES], sm.bc_hi, sm.bc_lo, tid - 32);   // warps 1 .. 3
-    }
-    const float4* Rr = sm.st.R[stage];
-    float(*part)[8] = sm.part[k & 1][warp];
-#pragma unroll 1
-    for (int h = 0; h < 2; ++h) {
-      uint32_t hw[2][3][4], lw[2][3][4];
-      const bool have = h * 8 < n;
-      const bool idle = have && __all_sync(0xffffffffu, !(T[0] > GS_T_STOP) && !(T[1] > GS_T_STOP));
-      if (have && !idle) {
-        float lr[2][8], lg[2][8], lb[2][8];
-        tmem_ld8x3(trow + h * 8, trow + 16 + h * 8, trow + 32 + h * 8, lr[0], lg[0], lb[0]);
-        tmem_ld8x3(trow + 48 + h * 8, trow + 64 + h * 8, trow + 80 + h * 8, lr[1], lg[1], lb[1]);
-        const float4* Rh = Rr + 32 * h;
-        float* ph = &part[h * 8][(lane >> 2) & 7];
-        const bool full = h * 8 + 8 <= n;
-#pragma unroll
-        for (int jp = 0; jp < 4; ++jp) {
-          float dc[2][2][3];
-#pragma unroll
-          for (int u = 0; u < 2; ++u) {
-            const int jj = 2 * jp + u;
-#pragma unroll
-            for (int p = 0; p < 2; ++p) dc[u][p][0] = dc[u][p][1] = dc[u][p][2] = 0.f;
-            if (full || h * 8 + jj < n) {
-              float v[8];
-              const float l0[3] = {lr[0][jj], lg[0][jj], lb[0][jj]}, l1[3] = {lr[1][jj], lg[1][jj], lb[1][jj]};
-              pair2(Rh[4 * jj], Rh[4 * jj + 1], l0, l1, dc[u], v);
-              const float r = reduce8(v, lane);
-              if ((lane & 3) == 0) ph[jj * 8] = r;
-            }
-          }
-#pragma unroll
-          for (int p = 0; p < 2; ++p)
-#pragma unroll
-            for (int c = 0; c < 3; ++c) split_bf16x2(dc[0][p][c], dc[1][p][c], hw[p][c][jp], lw[p][c][jp]);
-        }
-      } else if (idle) {
-#pragma unroll
-        for (int p = 0; p < 2; ++p)
-#pragma unroll
-          for (int c = 0; c < 3; ++c)
-#pragma unroll
-            for (int q = 0; q < 4; ++q) hw[p][c][q] = lw[p][c][q] = 0u;
-        part[h * 8 + (lane >> 2)][lane & 3] = 0.f;
-        part[h * 8 + (lane >> 2)][4 + (lane & 3)] = 0.f;
-      }
-      if (h == 0 && n_prev > 0) {
-        gs_mbar_wait(&sm.mma2_bar, par_prev);
-        fence_after_sync();
-      }
-      if (have) {
-#pragma unroll
-        for (int p = 0; p < 2; ++p)
-#pragma unroll
-          for (int c = 0; c < 3; ++c) {
-            sm.dct[(c * 2 + h) * 256 + tid + 128 * p] = make_uint4(hw[p][c][0], hw[p][c][1], hw[p][c][2], hw[p][c][3]);
-            sm.dct[(6 + c * 2 + h) * 256 + tid + 128 * p] = make_uint4(lw[p][c][0], lw[p][c][1], lw[p][c][2], lw[p][c][3]);
-          }
-      }
-      if (h == 0 && n_prev > 0) epilogue(n_prev, sm.st.R[(k - 1) % STAGES]);
-    }
-    fence_smem_to_async();
-    fence_before_sync();
-    const bool done = __syncthreads_and(!(T[0] > GS_T_STOP) && !(T[1] > GS_T_STOP)) != 0;
-    const bool more = !done && k + 1 < nchunks;
-    if (warp == 0) {
-      if (elect_one()) {
-        fence_after_sync();
-        if (more) tc_issue_logits(tm, sm.img_hi, sm.img_lo, sm.bc_hi, sm.bc_lo, &sm.mma_bar);
-        constexpr uint32_t idesc2 = idesc_bf16(1, 1, 128, 32);
-        const uint32_t a0 = gs_smem_u32(sm.dct), b0 = gs_smem_u32(sm.img_hi);
-#pragma unroll
-        for (int s = 0; s < 16; ++s)
-          mma_bf16(tm + D2COL + (uint32_t)(s & 1) * 32u, smem_desc(a0 + s * 256, 128, 4096), smem_desc(b0 + s * 256, 128, 4096),
-                   idesc2, s >= 2);
-        mma_commit(&sm.mma2_bar);
-      }
-      __syncwarp();
-    }
-    // geometry rows: threads 96 .. 111 (warp 3), one instance each
-    if (tid >= 96 && tid < 96 + n) {
-      const int j = tid - 96;
-      float s[6];
-#pragma unroll
-      for (int u = 0; u < 6; ++u) s[u] = (sm.part[k & 1][0][j][u] + sm.part[k & 1][1][j][u]) + (sm.part[k & 1][2][j][u] + sm.part[k & 1][3][j][u]);
-      const float4 a = Rr[4 * j];
-      const float4 b4 = Rr[4 * j + 1];
-      const float4 cc = Rr[4 * j + 2];
-      const uint32_t rxy = __float_as_uint(cc.z), rwh = __float_as_uint(cc.w);
-      const uint32_t slot = __float_as_uint(Rr[4 * j + 3].x) + ((uint32_t)ty - (rxy >> 16)) * (rwh & 0xffffu) +
-                            ((uint32_t)tx - (rxy & 0xffffu));
-      float* out = grad_inst + (size_t)slot * GREC;
-      out[0] = GS_LN2 * (2.f * a.z * s[0] - a.w * s[1]);
-      out[1] = GS_LN2 * (2.f * b4.x * s[1] - a.w * s[0]);
-      out[2] = -GS_LN2 * s[2];
-      out[3] = GS_LN2 * s[3];
-      out[4] = -GS_LN2 * s[4];
-      out[5] = GS_LN2 * s[5];
-      row_epoch[slot] = epoch;
-    }
-    n_prev = n;
-    par_prev = (uint32_t)(k & 1);
-    st_prev = stage;
-    if (done) {
-      consumed = min(cnt, (k + 1) * TC_J);
-      break;
-    }
-    if (k + STAGES - 1 < nchunks) {
-      const int kn = k + STAGES - 1;
-      tc_gather<K, STAGES, true, NT>(sm.st, kn % STAGES, grec, rgb, ids, goff, start + kn * TC_J, min(TC_J, cnt - kn * TC_J),
-                                     tid);
-    }
-  }
-  __syncthreads();
-  if (n_prev > 0) {
-    gs_mbar_wait(&sm.mma2_bar, par_prev);
-    fence_after_sync();
-    epilogue(n_prev, sm.st.R[st_prev]);
-  }
-  asm volatile("cp.async.wait_all;" ::: "memory");
-  fence_before_sync();
-  __syncthreads();
-  if (warp == 0) tmem_dealloc<TCOLS>(tm);
-  if (tile_neff_b && tid == 0) tile_neff_b[tile] = consumed;
-}
-
 }  // namespace
 
 cudaError_t gs_launch_blend_sh_fwd_tc(const GsRec* grec, const float* rgb, const uint32_t* ids, int d,
@@ -899,23 +608,15 @@ cudaError_t gs_launch_blend_sh_bwd_tc(const GsRec* grec, const float* rgb, const
                                       const float* grad_image, float* grad_inst, int grad_is_final, const GsCrop& crop,
                                       uint32_t* row_epoch, uint32_t epoch, int* tile_neff_b, cudaStream_t st) {
   if (!row_epoch) return cudaErrorInvalidValue;   // unprocessed rows are left stale: the consumer needs the epoch tags
-  const bool two_px = (gs_tuning().sh_tc & 4) != 0;   // two pixels per thread (128 threads per tile)
 #define GS_SHB_TC(K)                                                                                                  \
   do {                                                                                                                \
     /* per device and cheap: set on every launch rather than cached in a process-wide flag */                        \
-    cudaError_t e = two_px ? cudaFuncSetAttribute(blend_sh_bwd_tc2_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                                  (int)sizeof(TcBwdSmem<K>))                                          \
-                           : cudaFuncSetAttribute(blend_sh_bwd_tc_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                                  (int)sizeof(TcBwdSmem<K>));                                         \
+    cudaError_t e = cudaFuncSetAttribute(blend_sh_bwd_tc_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
+                                         (int)sizeof(TcBwdSmem<K>));                                                  \
     if (e != cudaSuccess) return e;                                                                                   \
-    if (two_px)                                                                                                       \
-      blend_sh_bwd_tc2_kernel<K><<<g.n_tiles, 128, sizeof(TcBwdSmem<K>), st>>>(                                        \
-          grec, rgb, ids, goff, tile_accum, g.wp, g.hp, g.ntx, g.fx, g.fy, r.rays_o, r.lefttop, r.dx, r.dy, image,     \
-          grad_image, grad_inst, grad_is_final, crop, row_epoch, epoch, tile_neff_b);                                 \
-    else                                                                                                              \
-      blend_sh_bwd_tc_kernel<K><<<g.n_tiles, TC_NT, sizeof(TcBwdSmem<K>), st>>>(                                        \
-          grec, rgb, ids, goff, tile_accum, g.wp, g.hp, g.ntx, g.fx, g.fy, r.rays_o, r.lefttop, r.dx, r.dy, image,     \
-          grad_image, grad_inst, grad_is_final, crop, row_epoch, epoch, tile_neff_b);                                 \
+    blend_sh_bwd_tc_kernel<K><<<g.n_tiles, TC_NT, sizeof(TcBwdSmem<K>), st>>>(                                          \
+        grec, rgb, ids, goff, tile_accum, g.wp, g.hp, g.ntx, g.fx, g.fy, r.rays_o, r.lefttop, r.dx, r.dy, image,       \
+        grad_image, grad_inst, grad_is_final, crop, row_epoch, epoch, tile_neff_b);                                   \
   } while (0)
   if (d == 27) GS_SHB_TC(9); else GS_SHB_TC(16);
 #undef GS_SHB_TC

@@ -100,25 +100,9 @@ __device__ __forceinline__ void gs_mbar_wait(uint64_t* bar, uint32_t parity) {
   } while (!ok);
 }
 
-__device__ __forceinline__ void gs_mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(gs_smem_u32(bar)) : "memory");
-}
-// named barriers over a SUBSET of the CTA's warps (the consumer warps of a warp-specialised kernel;
-// the producer warp never joins them).  `n` = number of participating threads (multiple of 32).
+// named barrier over a SUBSET of the CTA's warps.  `n` = number of participating threads (multiple of 32).
 __device__ __forceinline__ void gs_bar_sync(int id, int n) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory");
-}
-__device__ __forceinline__ int gs_bar_red_and(int id, int n, int pred) {
-  int r;
-  asm volatile(
-      "{\n\t.reg .pred p, q;\n\t"
-      "setp.ne.s32 p, %3, 0;\n\t"
-      "bar.red.and.pred q, %1, %2, p;\n\t"
-      "selp.s32 %0, 1, 0, q;\n\t}"
-      : "=r"(r)
-      : "r"(id), "r"(n), "r"(pred)
-      : "memory");
-  return r;
 }
 
 // pixel centre in normalised image-plane units, gaussian.cu:839-840 (double arithmetic,

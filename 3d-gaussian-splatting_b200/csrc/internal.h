@@ -46,21 +46,9 @@ struct GsRayPtrs {
   const float *rays_o, *lefttop, *dx, *dy;
 };
 
-// Run-time tuning knobs (A/B experiments and profiles/; the defaults are the shipped configuration).
-// Set with gs_tune("name", value) or the environment variable GS_TUNE_<NAME> (read once).
+// Run-time tuning knobs (the defaults are the shipped configuration).  Set with gs_tune("name", value) or the
+// environment variable GS_TUNE_<NAME> (read once; an out-of-range value there keeps the default).
 struct GsTuning {
-  int fwd_kernel;   // 0 = consumer thread 0 issues the copies, 1 = dedicated producer warp
-  int fwd_ch;       // staging chunk of kernel 0: 64 / 128 / 256
-  int bwd_kernel;   // 0 = shuffle-network reduction (round 1), 1 = two-phase shared-memory reduction
-  int bwd_px;       // pixels per consumer thread: 4 or 8
-  int bwd_ws;       // dedicated producer warp
-  int bwd_unroll;   // instances per unrolled step: 1, 2, 4
-  int bwd_stages;   // staging ring depth: 2 or 3
-  int bwd_minb;     // __launch_bounds__ min blocks (register cap); 1 = none
-  int bwd_rq;       // reducer threads per instance in the second phase: 4 (16 instances per round) or 8 (8)
-  int fwd_px;       // pixels per thread of forward kernel 0: 4 (2 warps per tile) or 8 (1 warp)
-  int bwd_ch;       // gather path: instances per staging chunk of the backward (64 or 32)
-  int strict;       // 1: an un-instantiated knob combination is an error (sweeps); 0: falls back to the shipped kernel
   int gather;       // fused frame path (RGB and SH): 1 = no pack pass, blend kernels gather records from rec[N]; 0 = packed streams
   int sh_tc;        // SH blend on the tensor cores (blend_sh_tc.cu, gather path only): bit 0 = forward, bit 1 = backward
 };
@@ -153,8 +141,7 @@ cudaError_t gs_launch_blend_bwd(const float4* pA, const float2* pB, const float4
                                 uint32_t epoch, int* tile_neff_b /*nullable: instances the backward consumed per tile*/,
                                 cudaStream_t st);
 
-// Maps frame (gather path, fixed configuration: the gs_tune knobs do not apply).  The backward additionally writes
-// d/d depth_i = sum g_D w into float 9 of every gradient row.
+// Maps frame (gather path).  The backward additionally writes d/d depth_i = sum g_D w into float 9 of every gradient row.
 cudaError_t gs_launch_blend_fwd_maps(const GsRec* grec, const uint32_t* ids, const int* tile_accum, const GsFrameGeom& g,
                                      float* image, int* tile_neff, float* final_img, const GsCrop& crop,
                                      const GsMapsFwd& maps, cudaStream_t st);

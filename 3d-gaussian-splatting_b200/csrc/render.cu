@@ -40,42 +40,41 @@ int gs_set_error_msg(int code, const char* what) {
 extern "C" const char* gs_last_error(void) { return g_err; }
 extern "C" int gs_abi_version(void) { return 2; }
 
-static int tune_env(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
+static int tune_env(const char* env, int dflt, int max) {
+  const char* e = getenv(env);
+  const int v = e ? atoi(e) : dflt;
+  return v >= 0 && v <= max ? v : dflt;
 }
 GsTuning& gs_tuning() {
-  // shipped configuration = the best of the sweeps in profiles/r2_sweeps.md
-  static GsTuning t = {tune_env("GS_TUNE_FWD_KERNEL", 0),  tune_env("GS_TUNE_FWD_CH", 128),   tune_env("GS_TUNE_BWD_KERNEL", 1),
-                       tune_env("GS_TUNE_BWD_PX", 8),      tune_env("GS_TUNE_BWD_WS", 0),     tune_env("GS_TUNE_BWD_UNROLL", 4),
-                       tune_env("GS_TUNE_BWD_STAGES", 3),  tune_env("GS_TUNE_BWD_MINB", 10),  tune_env("GS_TUNE_BWD_RQ", 4),
-                       tune_env("GS_TUNE_FWD_PX", 4),      tune_env("GS_TUNE_BWD_CH", 32),    tune_env("GS_TUNE_STRICT", 0),
-                       tune_env("GS_TUNE_GATHER", 1),      tune_env("GS_TUNE_SH_TC", 3)};
+  static GsTuning t = {tune_env("GS_TUNE_GATHER", 1, 1), tune_env("GS_TUNE_SH_TC", 3, 3)};
   return t;
 }
-static int* tune_knob(const char* name) {
+// the knob called `name` (nullptr if there is none) and its largest valid value; every range starts at 0
+static int* tune_knob(const char* name, int& max) {
   GsTuning& t = gs_tuning();
-  struct { const char* k; int* v; } tab[] = {{"fwd_kernel", &t.fwd_kernel}, {"fwd_ch", &t.fwd_ch},
-                                             {"bwd_kernel", &t.bwd_kernel}, {"bwd_px", &t.bwd_px},
-                                             {"bwd_ws", &t.bwd_ws},         {"bwd_unroll", &t.bwd_unroll},
-                                             {"bwd_stages", &t.bwd_stages}, {"bwd_minb", &t.bwd_minb},
-                                             {"bwd_rq", &t.bwd_rq},         {"fwd_px", &t.fwd_px},
-                                             {"gather", &t.gather},         {"bwd_ch", &t.bwd_ch},
-                                             {"strict", &t.strict},         {"sh_tc", &t.sh_tc}};
-  for (auto& e : tab)
-    if (!strcmp(e.k, name)) return e.v;
+  if (!strcmp(name, "gather")) {
+    max = 1;
+    return &t.gather;
+  }
+  if (!strcmp(name, "sh_tc")) {
+    max = 3;
+    return &t.sh_tc;
+  }
   return nullptr;
 }
 extern "C" int gs_tune(const char* name, int value) {
   if (!name) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_tune: null name");
-  int* v = tune_knob(name);
+  int max = 0;
+  int* v = tune_knob(name, max);
   if (!v) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_tune: unknown knob");
+  if (value < 0 || value > max) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_tune: value out of range");
   *v = value;
   return 0;
 }
 extern "C" int gs_tune_get(const char* name, int* value) {
   if (!name || !value) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_tune_get: null argument");
-  const int* v = tune_knob(name);
+  int max = 0;
+  const int* v = tune_knob(name, max);
   if (!v) return gs_set_error_msg(GS_ERR_INVALID_ARG, "gs_tune_get: unknown knob");
   *value = *v;
   return 0;

@@ -33,10 +33,13 @@ typedef void* gs_stream_t; /* cudaStream_t */
 int gs_abi_version(void);
 /* Human-readable text of the last error on this host thread ("" if none). */
 const char* gs_last_error(void);
-/* A/B tuning knobs of the blend kernels (profiles/ experiments; defaults = the shipped configuration):
- * "fwd_kernel", "fwd_ch", "bwd_kernel", "bwd_px", "bwd_ws", "bwd_unroll", "bwd_stages", "bwd_minb"
- * (see csrc/internal.h GsTuning).  An unsupported combination makes the next backward fail with
- * cudaErrorInvalidValue.  Process-wide, not thread-safe. */
+/* Blend-path knobs (defaults = the shipped configuration; environment GS_TUNE_GATHER / GS_TUNE_SH_TC, read once):
+ *   "gather"  1 (default) = the fused frame's blend kernels gather records through the sorted id list;
+ *             0 = a pack pass writes record streams first (the legacy draw API's kernels)
+ *   "sh_tc"   0..3, default 3: SH blend of the gather path on the tensor cores, bit 0 = forward, bit 1 = backward
+ *             (0 = the scalar kernels)
+ * An unknown name or a value out of range returns GS_ERR_INVALID_ARG and leaves the knob unchanged.
+ * Process-wide, not thread-safe. */
 int gs_tune(const char* name, int value);
 /* New: current value of a gs_tune knob (e.g. to restore it after an experiment). */
 int gs_tune_get(const char* name, int* value);
@@ -198,8 +201,7 @@ int gs_render_backward_final(gs_ctx* ctx, const float* pos, const float* rgb, co
  * three final pointers are set (all NULL or all set), image_final[height,width,3] = crop(clamp(image, 0, 1)),
  * depth_final / alpha_final[height,width] = crop(.) with NO clamp.  Same launches and one host synchronisation,
  * like gs_render_forward.  GS_ERR_UNSUPPORTED (reason in gs_last_error) for d != 3 (SH colour), with
- * gs_tune("gather", 0), and while a gs_ctx_set_grad_push configuration is active.  The A/B tuning knobs of the
- * blend kernels do not apply: a maps frame always runs the shipped gather configuration. */
+ * gs_tune("gather", 0), and while a gs_ctx_set_grad_push configuration is active. */
 int gs_render_forward_maps(gs_ctx* ctx, const float* pos, const float* rgb, const float* opa,
                            const float* quat, const float* scale, int n, int d, int scale_activation,
                            const gs_camera* cam_host, const float* background_host,

@@ -122,9 +122,10 @@ def test_argument_validation_needs_no_gpu():
     assert lib.gs_adam_step(0x1000, 0x2000, 0x3000, 0x4000, 16, ends, lrs, 9, 0.9, 0.99, 1e-8, 1, None) == -1  # > 8 segments
 
 
-def test_round2_entry_points_validate_without_a_gpu():
+def test_round2_entry_points_and_tune_knobs_validate_without_a_gpu():
     """The entry points added in round 2 (loss, densification, tuning, push-finish through the switch, launch
-    counter) reject bad arguments before touching CUDA."""
+    counter) reject bad arguments before touching CUDA; gs_tune knows exactly the knobs gather and sh_tc and
+    refuses values outside their ranges."""
     lib = ctypes.CDLL(os.path.join(PKG, "libgs_b200.so"))
     lib.gs_last_error.restype = ctypes.c_char_p
     P, LL, I, F = ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int, ctypes.c_float
@@ -150,9 +151,27 @@ def test_round2_entry_points_validate_without_a_gpu():
     lib.gs_tune.argtypes = [ctypes.c_char_p, I]
     assert lib.gs_tune(b"no_such_knob", 1) == -1 and "unknown knob" in err()
     assert lib.gs_tune(None, 1) == -1
-    # every documented knob is accepted (values are validated at launch time); restore the shipped defaults
-    for knob, dflt in ((b"sh_tc", 3), (b"gather", 1), (b"strict", 0), (b"bwd_ch", 32)):
-        assert lib.gs_tune(knob, dflt) == 0, knob
+    lib.gs_tune_get.argtypes = [ctypes.c_char_p, ctypes.POINTER(I)]
+
+    def tuned(knob):
+        v = I(-1)
+        assert lib.gs_tune_get(knob, ctypes.byref(v)) == 0, knob
+        return v.value
+
+    # the two knobs accept every value of their range; the shipped defaults are restored last
+    for knob, values, dflt in ((b"gather", (0, 1), 1), (b"sh_tc", (0, 1, 2, 3), 3)):
+        for value in values + (dflt,):
+            assert lib.gs_tune(knob, value) == 0, (knob, value)
+            assert tuned(knob) == value
+    # out of range: refused, and the knob keeps its value
+    for knob, bad in ((b"sh_tc", 7), (b"sh_tc", -1), (b"gather", 2), (b"gather", -1)):
+        before = tuned(knob)
+        assert lib.gs_tune(knob, bad) == -1 and "out of range" in err(), (knob, bad)
+        assert tuned(knob) == before
+    # the knobs of the retired blend-kernel variants are gone
+    for knob in (b"fwd_kernel", b"fwd_ch", b"fwd_px", b"bwd_kernel", b"bwd_px", b"bwd_ws", b"bwd_unroll", b"bwd_stages",
+                 b"bwd_minb", b"bwd_rq", b"bwd_ch", b"strict"):
+        assert lib.gs_tune(knob, 0) == -1 and "unknown knob" in err(), knob
     lib.gs_allreduce_push_finish_mc_f32.argtypes = [P, P, P, LL, LL, I, I, P]
     assert lib.gs_allreduce_push_finish_mc_f32(None, 0x1000, 0x2000, 64, 32, 0, 2, None) == -1
     assert lib.gs_allreduce_push_finish_mc_f32(0x1000, 0x2000, 0x3000, 64, 16, 0, 2, None) == -1      # 2 * per < n
